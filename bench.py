@@ -42,7 +42,30 @@ def parse():
     ap.add_argument('--no-cpu-baseline', action='store_true')
     ap.add_argument('--no-graph', action='store_true')
     ap.add_argument('--no-extra', action='store_true', help='skip the cfg1 / cfg3 side measurements')
-    return ap.parse_args()
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='write the loss, log-probs and output lengths of the last timed train step to DIR/<name>.npy')
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    return args
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """Write each array as out_dir/<name>.npy in float32 / float64.  An array larger than its share of DUMP_LIMIT_BYTES is
+    replaced by a fixed sample of its elements (same positions for the same shape), so two builds compare element for
+    element."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    share = DUMP_LIMIT_BYTES // len(arrays)
+    for name, a in arrays.items():
+        a = np.asarray(a)
+        if a.itemsize * a.size > share:
+            idx = np.random.default_rng(0).choice(a.size, share // a.itemsize, replace=False)
+            a = a.reshape(-1)[np.sort(idx)]
+        np.save(os.path.join(out_dir, f'{name}.npy'), a)
 
 
 def peaks():
@@ -260,8 +283,16 @@ def main():
     sampler = ClockSampler(local)
     if rank == 0:
         sampler.start()
-    ms = timed(lambda: tr.step(dev_batch, training=True), args.steps, max(3, args.warmup), eng)
+    last = {}
+
+    def train_step():
+        last['out'] = tr.step(dev_batch, training=True)
+    ms = timed(train_step, args.steps, max(3, args.warmup), eng)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        loss, logp, out_len = last['out']
+        dump_outputs(args.dump_outputs, {'loss': loss.double().cpu().numpy(), 'log_probs': logp.float().cpu().numpy(),
+                                         'out_len': out_len.double().cpu().numpy()})
     launches_total = timed.launches
     ms_step = ms / args.steps
     value = world * B * args.steps / (ms / 1e3)
@@ -300,8 +331,8 @@ def main():
         cfg3 = {}
         for name in ('c7d2_skips', 'linear_skips'):
             m3, t3, _, db3 = build(ARCHS[name], args.precision, B, T)
-            ms3 = timed(lambda: t3.step(db3, training=True), max(5, args.steps // 2), 3, m3.engine)
-            n3 = max(5, args.steps // 2)
+            n3 = args.steps
+            ms3 = timed(lambda: t3.step(db3, training=True), n3, 3, m3.engine)
             cfg3[name] = {'arch_vec': ARCHS[name], 'ms_per_step': ms3 / n3, 'value': world * B * n3 / (ms3 / 1e3), 'unit': 'utt/s',
                           'grad_bytes_per_step': 4 * int(m3.engine.n_flat), 'gpu_launches_per_step': timed.launches / n3}
             del m3, t3, db3
@@ -358,12 +389,13 @@ def cfg1_entry(args, torch, nb, build, timed, dev):
             loss, logp, ol = t1.step(db, training=False)
             state['loss'] = loss
             return t1.decode(logp, ol, db)
-        ms1 = timed(ev, 20, 3, m1.engine)
+        n1 = args.steps
+        ms1 = timed(ev, n1, 3, m1.engine)
         per = ev()
         audio_s = float(hb[0][1].sum()) / 100.0
         res[prec] = dict(loss=float(state['loss'].item()), per=float(per.item()), dist=t1.last_hyp[2].cpu().tolist())
-        out[f'gpu_{prec}'] = {'value': audio_s * 20 / (ms1 / 1e3), 'unit': 'audio-s/s', 'ms_per_step': ms1 / 20,
-                              'utt_per_s': B1 * 20 / (ms1 / 1e3)}
+        out[f'gpu_{prec}'] = {'value': audio_s * n1 / (ms1 / 1e3), 'unit': 'audio-s/s', 'ms_per_step': ms1 / n1,
+                              'utt_per_s': B1 * n1 / (ms1 / 1e3)}
         del m1, t1
         torch.cuda.empty_cache()
     if not args.no_cpu_baseline:
