@@ -193,6 +193,9 @@ int nbasr_layernorm_bwd(int dtype, const void* dy, const void* x, int x_dtype, f
 
 /* (B, F, T) fp32 channel-first input (trainer.py:210) -> padded channels-last (B, Tp, F), multiplied by `scale`. */
 int nbasr_transpose_in(const float* audio, void* out, int dtype, int B, int F, int T, int Tp, float scale, void* stream);
+/* The inverse: padded channels-last fp32 (B, Tp, F), frame t at row b*Tp + PAD_L + t -> (B, F, T) fp32 (the input
+ * gradient of the model). */
+int nbasr_transpose_out(const float* in, float* out, int B, int F, int T, int Tp, void* stream);
 
 /* Weight packing: out[n][q*M + m] = w[m*ws_m + n*ws_n + (t0 + q*tstep)*ws_t],  q < nq.
  * Produces the bf16 / fp32 operand copies (plain, transposed, tap-flipped) used by gemm_tn. */
@@ -271,6 +274,18 @@ int nbasr_beam_per(const float* logp, int B, int T, int V, const int64_t* audio_
 int nbasr_optim_step(float* param, float* grad, float* m, float* v, int64_t n, const int64_t* seg_off,
                      const int64_t* seg_len, int nseg, int64_t seg_chunks, float reg_coef, float max_norm,
                      float beta1, float beta2, float eps, float* state, void* stream);
+
+/* Per-tensor statistics of the zero-cost architecture proxies over the same flat fp32 buffers and segment table format as
+ * nbasr_optim_step: out[2*s] = sum g^2 and out[2*s + 1] = sum |param * grad| over segment s, products and sums in fp64.
+ * part: 2 * seg_chunks doubles of scratch.  Deterministic: fixed 16384-element chunks, partials summed in chunk order. */
+int nbasr_param_stats(const float* param, const float* grad, const int64_t* seg_off, const int64_t* seg_len, int nseg,
+                      int64_t seg_chunks, double* part, double* out, void* stream);
+
+/* Row Gram matrix and row sums of a (B, D) fp32 matrix with row pitch ld (B <= 128), in fp64:
+ * gram[i*B + j] = sum_d x[i*ld + d] * x[j*ld + d],  rowsum[i] = sum_d x[i*ld + d].
+ * work: ceil(D / 256) * (B*(B+1)/2 + B) doubles.  Deterministic (256-column chunks summed in chunk order).
+ * Used on a padded channels-last input gradient (ld = D = Tp*C): its zero pad rows add nothing. */
+int nbasr_row_gram(const float* x, int B, int64_t D, int64_t ld, double* gram, double* rowsum, double* work, void* stream);
 
 /* Batched operand refresh: ONE launch executes a device-resident table of pack jobs (what
  * nbasr_convert / nbasr_pack_weight / nbasr_pack_gconv_mma / nbasr_pack_gconv_dgrad do one at a time).

@@ -55,6 +55,9 @@ _SIGS = {
     'nbasr_layernorm_bwd': [C.c_int, _vp, _vp, C.c_int, _f32, _vp, _vp, _vp, C.c_int, C.c_int, C.c_int, C.c_int, _vp, _vp, _vp,
                             _f32, _i64, C.c_int, _vp, _vp, _vp],
     'nbasr_transpose_in': [_vp, _vp, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _f32, _vp],
+    'nbasr_transpose_out': [_vp, _vp, C.c_int, C.c_int, C.c_int, C.c_int, _vp],
+    'nbasr_param_stats': [_vp, _vp, _vp, _vp, C.c_int, _i64, _vp, _vp, _vp],
+    'nbasr_row_gram': [_vp, C.c_int, _i64, _i64, _vp, _vp, _vp, _vp],
     'nbasr_pack_weight': [_vp, _vp, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _i64, _i64, _i64, _vp],
     'nbasr_convert': [_vp, _vp, C.c_int, _i64, _vp],
     'nbasr_lstm_fwd': [_vp, _vp, C.c_int, C.c_int, C.c_int, _vp, C.c_int, _i64, _i64, _i64, _vp, _vp, _vp, _vp, _vp],

@@ -236,6 +236,22 @@ __global__ void transpose_in_kernel(const float* __restrict__ a, T* __restrict__
   }
 }
 
+// the inverse layout change: padded channels-last fp32 (B, Tp, F) -> (B, F, T) fp32
+__global__ void transpose_out_kernel(const float* __restrict__ in, float* __restrict__ out, int B, int F, int Tt, int Tp) {
+  __shared__ float tile[32][33];
+  int b = blockIdx.z;
+  int t0 = blockIdx.x * 32, f0 = blockIdx.y * 32;
+  for (int i = threadIdx.y; i < 32; i += blockDim.y) {
+    int t = t0 + i, f = f0 + threadIdx.x;
+    tile[i][threadIdx.x] = (t < Tt && f < F) ? in[((int64_t)b * Tp + NBASR_PAD_L + t) * F + f] : 0.f;
+  }
+  __syncthreads();
+  for (int i = threadIdx.y; i < 32; i += blockDim.y) {
+    int f = f0 + i, t = t0 + threadIdx.x;
+    if (f < F && t < Tt) out[((int64_t)b * F + f) * Tt + t] = tile[threadIdx.x][i];
+  }
+}
+
 template <typename T>
 __global__ void pack_weight_kernel(const float* __restrict__ w, T* __restrict__ out, int M, int N, int nq, int t0,
                                    int tstep, int64_t ws_m, int64_t ws_n, int64_t ws_t) {
@@ -337,6 +353,14 @@ int nbasr_transpose_in(const float* audio, void* out, int dtype, int B, int F, i
   if (dtype == NBASR_BF16) transpose_in_kernel<bf16><<<grid, block, 0, as_stream(stream)>>>(audio, (bf16*)out, B, F, T, Tp, scale);
   else if (dtype == NBASR_F16) transpose_in_kernel<f16><<<grid, block, 0, as_stream(stream)>>>(audio, (f16*)out, B, F, T, Tp, scale);
   else transpose_in_kernel<float><<<grid, block, 0, as_stream(stream)>>>(audio, (float*)out, B, F, T, Tp, scale);
+  NBASR_CHECK_LAUNCH();
+  return 0;
+}
+
+int nbasr_transpose_out(const float* in, float* out, int B, int F, int T, int Tp, void* stream) {
+  if (B <= 0 || F <= 0 || T <= 0) return 0;
+  dim3 grid((T + 31) / 32, (F + 31) / 32, B), block(32, 8);
+  transpose_out_kernel<<<grid, block, 0, as_stream(stream)>>>(in, out, B, F, T, Tp);
   NBASR_CHECK_LAUNCH();
   return 0;
 }

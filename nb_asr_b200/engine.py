@@ -445,22 +445,25 @@ class Engine:
         e.accumulate = accumulate
         return e
 
-    def plan(self, B, T, training, grad=None):
-        """Plans are cached per (B, T, training, grad), least recently used first.  `training` switches dropout on; `grad`
-        (default: training) says whether a backward pass may follow: only then are gate-bit masks, bf16 twins of the
-        forward activations and the backward call list built (an eval step needs none of them).  A plan owns every activation / mask /
-        gradient buffer of its shape (about 3.7 GB at 64 x 500) plus the CUDA graphs and CTC workspaces captured on it, so
+    def plan(self, B, T, training, grad=None, input_grad=False):
+        """Plans are cached per (B, T, training, grad[, 'input_grad']), least recently used first.  `training` switches
+        dropout on; `grad` (default: training) says whether a backward pass may follow: only then are gate-bit masks, bf16
+        twins of the forward activations and the backward call list built (an eval step needs none of them).  `input_grad`
+        (implies grad) appends the gradient wrt the input features to the backward pass: pl.daudio (B, 80, T) fp32.  A plan
+        owns every activation / mask / gradient buffer of its shape (about 3.7 GB at 64 x 500) plus the CUDA graphs and CTC workspaces captured on it, so
         loaders whose padded length changes from batch to batch would otherwise grow without bound: beyond `max_plans`
         (NBASR_MAX_PLANS, default 6) the oldest plan is dropped and its memory returns to the allocator."""
         grad = bool(training) if grad is None else bool(grad)
-        key = (B, T, bool(training), grad)
+        input_grad = bool(input_grad)
+        grad = grad or input_grad
+        key = (B, T, bool(training), grad) + (('input_grad',) if input_grad else ())
         pl = self.plans.get(key)
         if pl is None:
             while len(self.plans) >= max(1, self.max_plans):
                 _, old = self.plans.popitem(last=False)
                 old.graphs.clear()
                 old.ws.clear()
-            pl = self.plans[key] = self._build_plan(B, T, bool(training), grad)
+            pl = self.plans[key] = self._build_plan(B, T, bool(training), grad, input_grad)
         else:
             self.plans.move_to_end(key)
         return pl
@@ -482,12 +485,12 @@ class Engine:
         return int(total * 1.05) + (8 << 20)
 
     @_on_device
-    def _build_plan(self, B, T, training, grad=True):
+    def _build_plan(self, B, T, training, grad=True, input_grad=False):
         self.bind()
         m, lib, dev, dt, tdt = self.model, self.lib, self.device, self.dt, self.tdt
         es = 2 if dt == BF16 else 4
         pl = _Plan()
-        pl.B, pl.T, pl.training, pl.grad = B, T, training, grad
+        pl.B, pl.T, pl.training, pl.grad, pl.input_grad = B, T, training, grad, input_grad
         pl.keep = []       # keeps ctypes structs / tensors alive
         pl.graphs, pl.ws = {}, {}     # CUDA graphs / CTC workspaces captured on this plan (trainer.py); die with the plan
         arena = pl.arena = _Arena(dev, self._plan_bytes_estimate(B, T, grad))
@@ -885,6 +888,8 @@ class Engine:
                 gout = g[0]
             # ---- top of the block: LayerNorm bwd -> dZ of the time-reduction conv
             dzc = dz[0]
+            if i == 0:
+                dz_blk0 = dzc
             lname, cname = self.block_ln[i], self.block_conv[i]
             call(bwd, lib.nbasr_layernorm_bwd, dt, gout.data_ptr(), rec['z'].data_ptr(), adt, S, rec['mean'].data_ptr(),
                  rec['rstd'].data_ptr(), self.P(lname + '.weight'), B, Ti, Tp, Cc, None, dzc.data_ptr(), rec['zmask'].t.data_ptr(),
@@ -910,6 +915,25 @@ class Engine:
                         epi = self._epi(Cin, out=gout.data_ptr())
                         gemm(bwd, _ptr(dzc, (PAD_L - 1 + par) * Cc), Tp * Cc, Cc, B, nrp, 4 * Cc, Cin,
                              self.wd[cname][par].data_ptr(), 4 * Cc, PAD_L + par, pgeo.Tp, 2, epi)
+        pl.daudio = None
+        if input_grad:
+            # Gradient wrt the input features: block 0's stride-1 input-gradient GEMM (as for blocks > 0 above, C_in = 80),
+            # fp32 output into a padded (B, Tp, 80) buffer, then back to the (B, 80, T) layout of the input.  The tap-flipped
+            # operand of conv_0 belongs to this plan and is re-packed by it: the optimiser tail (and every CUDA graph
+            # captured on it) keeps refreshing exactly the packs it refreshes without input gradients.
+            rec = block_records[0]
+            geo, cname = rec['geo'], self.block_conv[0]
+            Cc, Tp = geo.C, geo.Tp
+            wd0 = arena.zeros((FEATURES, 8 * Cc), tdt)
+            call(bwd, lib.nbasr_pack_weight, self.P(cname + '.weight'), wd0.data_ptr(), dt, Cc, FEATURES, 8, 7, -1,
+                 8 * FEATURES, 1, FEATURES)
+            pl.dx_in = arena.zeros((g_in.rows, FEATURES), torch.float32)
+            epi = self._epi(FEATURES, out=pl.dx_in.data_ptr(), out_dtype=F32)
+            gemm(bwd, _ptr(dz_blk0, (PAD_L - 4) * Cc), Tp * Cc, Cc, B, T, 8 * Cc, FEATURES, wd0.data_ptr(), 8 * Cc, PAD_L,
+                 g_in.Tp, 1, epi)
+            pl.daudio = arena.zeros((B, FEATURES, T), torch.float32)
+            call(bwd, lib.nbasr_transpose_out, pl.dx_in.data_ptr(), pl.daudio.data_ptr(), B, FEATURES, T, g_in.Tp)
+            pl.in_geo = g_in
         pl.bwd = bwd
         return pl
 
@@ -927,13 +951,14 @@ class Engine:
         self.launches += n
 
     @_on_device
-    def forward(self, audio, training=None, grad=None):
-        """audio (B, 80, T) fp32 cuda -> plan (holds logits / logp buffers).  grad: a backward pass may follow."""
+    def forward(self, audio, training=None, grad=None, input_grad=False):
+        """audio (B, 80, T) fp32 cuda -> plan (holds logits / logp buffers).  grad: a backward pass may follow;
+        input_grad: it also computes pl.daudio, the gradient wrt `audio`."""
         self.bind()
         training = self.model.training if training is None else training
         B, F, T = audio.shape
         assert F == FEATURES
-        pl = self.plan(B, T, training, grad)
+        pl = self.plan(B, T, training, grad, input_grad)
         self.refresh_packs()
         pl.audio.copy_(audio, non_blocking=True)
         if training and self.training_drop > 0:
@@ -1001,8 +1026,9 @@ class ModelFunction(torch.autograd.Function):
         eng = model.engine
         # gradients may be requested in eval mode too (dropout off): the plan then still records gate masks
         need = torch.is_grad_enabled() and (audio.requires_grad or any(p.requires_grad for p in eng.params))
-        pl = eng.forward(audio.contiguous().float(), grad=need or model.training)
-        ctx.eng, ctx.pl = eng, pl
+        need_x = ctx.needs_input_grad[1]        # (grad mode is off inside Function.forward: ask autograd)
+        pl = eng.forward(audio.contiguous().float(), grad=need or model.training, input_grad=need_x)
+        ctx.eng, ctx.pl, ctx.audio_dtype = eng, pl, audio.dtype
         return pl.logits.clone()
 
     @staticmethod
@@ -1037,5 +1063,7 @@ class ModelFunction(torch.autograd.Function):
             else:
                 dst.view(p.shape).add_(g.detach().to(dst.device, torch.float32))
         eng.attach_grads()
-        # gradients were written in place into p.grad (views of the flat buffer)
-        return (None, None) + tuple(None for _ in eng.params)
+        # gradients were written in place into p.grad (views of the flat buffer); the input gradient is returned (autograd
+        # accumulates it into audio.grad)
+        daudio = pl.daudio.to(ctx.audio_dtype, copy=True) if pl.daudio is not None else None
+        return (None, daudio) + tuple(None for _ in eng.params)

@@ -21,10 +21,12 @@ import pickle
 from . import PhonemeEncoder, data, distributed, get_loss, get_model, get_trainer, graph_utils, search_space, set_seed
 
 
-def evaluate_arch(arch, batches, gpu, precision='bf16', seed=1235, init='reference', conv_gain=1.0, n_ref=None):
+def evaluate_arch(arch, batches, gpu, precision='bf16', seed=1235, init='reference', conv_gain=1.0, n_ref=None, proxies=(),
+                  proxy_batches=1):
     """One candidate: build from `seed`, eval step (forward + CTC loss) and greedy decode + PER on every batch.
     Returns the reference's epoch metrics (AvgMeter, trainer.py:16-33: unweighted mean of the per-batch means) plus the
-    corpus-level PER (sum of edit distances / sum of reference lengths)."""
+    corpus-level PER (sum of edit distances / sum of reference lengths), and for every measure in `proxies` its
+    zero-cost proxy score (nb_asr_b200.proxies) averaged over the first `proxy_batches` batches."""
     if init == 'reference':
         set_seed(seed)
     model = get_model(arch, use_rnn=True, dropout_rate=0.0, gpu=gpu, precision=precision, init=init, seed=seed, conv_gain=conv_gain)
@@ -40,15 +42,33 @@ def evaluate_arch(arch, batches, gpu, precision='bf16', seed=1235, init='referen
         pers.append(per.double())
         dists.append(tr.last_hyp[2].sum().double())
     res = torch.stack([torch.stack(losses).mean(), torch.stack(pers).mean(), torch.stack(dists).sum()]).tolist()
+    scores = {}
+    if proxies:
+        from .proxies import compute_proxies
+        use = batches[:max(1, proxy_batches)]
+        per_batch = [compute_proxies(model, b, proxies) for b in use]
+        scores = {m: sum(p[m] for p in per_batch) / len(per_batch) for m in proxies}
     model._engine = None
     row = dict(arch=arch, loss=res[0], per=res[1])
     if n_ref:
         row['per_corpus'] = res[2] / n_ref
+    row.update(scores)
     return row
 
 
-def main():
+def proxy_list(text):
+    """argparse type of --proxies: comma-separated measure names of nb_asr_b200.proxies.MEASURES."""
+    from .proxies import parse_measures
+    try:
+        return parse_measures(text)
+    except ValueError as e:
+        raise argparse.ArgumentTypeError(str(e)) from e
+
+
+def build_parser():
     ap = argparse.ArgumentParser()
+
+
     ap.add_argument('--limit', type=int, default=16, help='number of architectures (0 = the whole list)')
     ap.add_argument('--arch-file', default=None, help='JSON list of arch_vecs (e.g. the 8242 unique ones)')
     ap.add_argument('--dataset', default='timit', choices=['timit', 'uniform'],
@@ -69,7 +89,17 @@ def main():
     ap.add_argument('--out', default=None)
     ap.add_argument('--out-pickle', default=None, help='nb-asr style table: header, then rows')
     ap.add_argument('--all', action='store_true', help='evaluate every arch_vec, not one per isomorphism class')
-    args = ap.parse_args()
+    ap.add_argument('--proxies', type=proxy_list, default=(),
+                    help='comma-separated zero-cost proxies to add as columns: grad_norm,snip,synflow,jacob_cov')
+    ap.add_argument('--proxy-batches', type=int, default=1,
+                    help='the proxies are averaged over the first N batches of the evaluation set')
+    return ap
+
+
+def main():
+    args = build_parser().parse_args()
+    if args.proxy_batches < 1:
+        raise SystemExit('--proxy-batches must be >= 1')
     rank = int(os.environ.get('RANK', 0))
     world = int(os.environ.get('WORLD_SIZE', 1))
     local = int(os.environ.get('LOCAL_RANK', 0))
@@ -103,7 +133,8 @@ def main():
     t0 = time.time()
     rows = []
     for i in mine:
-        r = evaluate_arch(archs[i], batches, local, args.precision, seed=args.seed, init=args.init, conv_gain=args.conv_gain, n_ref=n_ref)
+        r = evaluate_arch(archs[i], batches, local, args.precision, seed=args.seed, init=args.init, conv_gain=args.conv_gain, n_ref=n_ref,
+                          proxies=args.proxies, proxy_batches=args.proxy_batches)
         r['index'] = i
         r['hash'] = graph_utils.get_model_hash(archs[i])
         rows.append(r)
@@ -129,12 +160,15 @@ def main():
             json.dump(dict(summary=summary, rows=rows), open(args.out, 'w'))
         if args.out_pickle:
             header = dict(dataset_type='b200-sweep-eval', version=2, search_space=search_space.get_search_space(),
-                          ops=search_space.all_ops, columns=['model_hash', 'arch_vec', 'ctc_loss', 'per', 'per_corpus'], seed=args.seed,
-                          precision=args.precision, dataset=args.dataset, utterances=n_utt, init=args.init,
+                          ops=search_space.all_ops, columns=['model_hash', 'arch_vec', 'ctc_loss', 'per', 'per_corpus'] + list(args.proxies),
+                          seed=args.seed, precision=args.precision, dataset=args.dataset, utterances=n_utt, init=args.init,
                           conv_gain=summary['conv_gain'], data='synthetic', decode='greedy')
+            if args.proxies:
+                header['proxy_batches'] = min(args.proxy_batches, len(batches))
             with open(args.out_pickle, 'wb') as f:
                 pickle.dump(header, f)
-                pickle.dump([[r['hash'], r['arch'], r['loss'], r['per'], r.get('per_corpus')] for r in rows], f)
+                pickle.dump([[r['hash'], r['arch'], r['loss'], r['per'], r.get('per_corpus')] + [r[m] for m in args.proxies]
+                             for r in rows], f)
     if world > 1:
         torch.distributed.destroy_process_group()
 
