@@ -287,6 +287,27 @@ int nbasr_param_stats(const float* param, const float* grad, const int64_t* seg_
  * Used on a padded channels-last input gradient (ld = D = Tp*C): its zero pad rows add nothing. */
 int nbasr_row_gram(const float* x, int B, int64_t D, int64_t ld, double* gram, double* rowsum, double* work, void* stream);
 
+/* One ReLU layer of the NASWOT proxy: a gate-bit mask in the plane-major format of nbasr_epilogue (mask_out) over the
+ * padded rows of one encoder block; frame t of utterance b is row b*Tp + NBASR_PAD_L + t. */
+typedef struct nbasr_gate_layer {
+  const void* mask;
+  int64_t mask_rows;    /* rows per plane */
+  int32_t w;            /* plane width: 32 (4-byte entries), 40 or 48 (8-byte entries) */
+  int32_t C;            /* channels: columns >= C of the last plane and bits >= w of an entry are ignored */
+  int32_t Tp;           /* rows per utterance */
+  int32_t T;            /* frames of the block */
+  int32_t s;            /* valid frames of utterance b: L = min(T, ceil(audio_len[b] / 2^s)) */
+  int32_t reserved;
+} nbasr_gate_layer;
+
+/* NASWOT kernel matrix (Mellor et al. 2021) over gate bits m = (0 < z <= relu_hi):
+ *   K[i*B + j] = sum over layers, frames t < min(L_i, L_j), channels c < C of [m_i(t, c) == m_j(t, c)]   (both triangles).
+ * layers: DEVICE array of nlayers (<= 1024) entries; audio_len (B) int64; 1 <= B <= 128 (larger B is an error).
+ * work: nbasr_gate_gram_work_elems(B) uint64.  Exact integer sums: deterministic.  Every entry of K is written. */
+int nbasr_gate_gram(const nbasr_gate_layer* layers, int nlayers, const int64_t* audio_len, int B, uint64_t* K,
+                    uint64_t* work, void* stream);
+int64_t nbasr_gate_gram_work_elems(int B);
+
 /* Batched operand refresh: ONE launch executes a device-resident table of pack jobs (what
  * nbasr_convert / nbasr_pack_weight / nbasr_pack_gconv_mma / nbasr_pack_gconv_dgrad do one at a time).
  * jobs: device array of n nbasr_pack_job; blockmap: device int32 pairs (job, chunk), one per thread block.  A chunk is

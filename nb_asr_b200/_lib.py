@@ -39,6 +39,11 @@ class GConv(C.Structure):
                 ('ktaps', _i32), ('off0', _i32), ('dstep', _i32), ('w', _vp), ('w_packed', _i32), ('epi', Epilogue)]
 
 
+class GateLayer(C.Structure):
+    _fields_ = [('mask', _vp), ('mask_rows', _i64), ('w', _i32), ('C', _i32), ('Tp', _i32), ('T', _i32), ('s', _i32),
+                ('reserved', _i32)]
+
+
 _SIGS = {
     'nbasr_gemm_tn': [C.POINTER(Gemm), _vp],
     'nbasr_gemm_wgrad': [C.POINTER(Wgrad), _vp],
@@ -58,6 +63,8 @@ _SIGS = {
     'nbasr_transpose_out': [_vp, _vp, C.c_int, C.c_int, C.c_int, C.c_int, _vp],
     'nbasr_param_stats': [_vp, _vp, _vp, _vp, C.c_int, _i64, _vp, _vp, _vp],
     'nbasr_row_gram': [_vp, C.c_int, _i64, _i64, _vp, _vp, _vp, _vp],
+    'nbasr_gate_gram': [_vp, C.c_int, _vp, C.c_int, _vp, _vp, _vp],
+    'nbasr_gate_gram_work_elems': [C.c_int],
     'nbasr_pack_weight': [_vp, _vp, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _i64, _i64, _i64, _vp],
     'nbasr_convert': [_vp, _vp, C.c_int, _i64, _vp],
     'nbasr_lstm_fwd': [_vp, _vp, C.c_int, C.c_int, C.c_int, _vp, C.c_int, _i64, _i64, _i64, _vp, _vp, _vp, _vp, _vp],
@@ -112,6 +119,7 @@ def load():
     lib.nbasr_gconv_mma_pack_elems.restype = C.c_int64
     lib.nbasr_gconv_chain_work_bytes.restype = C.c_int64
     lib.nbasr_logmel_work_floats.restype = C.c_int64
+    lib.nbasr_gate_gram_work_elems.restype = C.c_int64
     lib.nbasr_last_error.restype = C.c_char_p
     lib.nbasr_last_error.argtypes = []
     _lib = lib

@@ -575,6 +575,9 @@ class Engine:
         Tcur = T
         arch = m.arch_desc
         pl.block_geo = []
+        # ReLU20 layers of a grad plan in forward order, (gate mask, block geometry, block index): what the NASWOT proxy
+        # reads (proxies.nwot_kernel).  The block convs' and the non-`zero` node ops' masks; nothing else carries one.
+        pl.gates = [] if grad else None
         # backward bookkeeping: per block a pool of gradient buffers
         gpools = []
         block_records = []
@@ -590,6 +593,8 @@ class Engine:
             z = zact(geo.rows, Cc)
             zmask = _Mask(geo.rows, Cc, 32, arena) if grad else None     # gate bits are only read by the backward pass
             pl.keep.append(zmask)
+            if grad:
+                pl.gates.append((zmask, geo, i))
             wf_ptr = self.wf[cname].data_ptr() if self.wf[cname] is not None else self.P(cname + '.weight')
             a_ptr = _ptr(prev, (PAD_L - lpad) * pg.C)
             a_ptr_b = _ptr(Bc(prev), (PAD_L - lpad) * pg.C)      # the same rows of the bf16 copy (weight gradient)
@@ -632,6 +637,8 @@ class Engine:
                         mask = _Mask(geo.rows, Cc, mwid, arena) if grad else None
                         pl.keep.append(mask)
                         nrec['mask'] = mask
+                        if grad:
+                            pl.gates.append((mask, geo, i))
                         sl = next_salt()
                         if op == 'linear':
                             epi = self._epi(Cc, bias=self.P(pn + '.linear.bias'), relu=1, drop_p=drop_p, salt=sl, adds=adds,

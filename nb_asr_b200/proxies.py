@@ -1,14 +1,22 @@
 """Zero-cost architecture proxies: scores of an UNTRAINED candidate from one minibatch (pruning-at-init measures, as the
 NAS-Bench-ASR users' proxy code computes them through ``get_prunable_copy``).
 
-    compute_proxies(model, batch) -> {'grad_norm': ..., 'snip': ..., 'synflow': ..., 'jacob_cov': ...}
+    compute_proxies(model, batch) -> {'grad_norm': ..., 'snip': ..., 'synflow': ..., 'jacob_cov': ..., 'nwot': ...}
 
 * grad_norm = sum over scored tensors of ||g||_2 and snip = sum |theta * g|, from ONE forward + backward of the CTC loss
   (get_loss() on the log-softmax logits, output_len = audio_len // 4, no regulariser, dropout off);
 * jacob_cov: backward of dlogits = 1, the input gradient J (B, 80*T), score -sum(log(l + 1e-5) + 1 / (l + 1e-5)) over the
   eigenvalues l of corrcoef(J); NaN when a row of J has zero variance;
 * synflow: on the norm-free copy (get_prunable_copy(bn=False)) in the fp32 engine mode, every parameter replaced by its
-  absolute value, an all-ones (1, 80, T) input, dlogits = 1; score sum |theta * g|.
+  absolute value, an all-ones (1, 80, T) input, dlogits = 1; score sum |theta * g|;
+* nwot (NASWOT, Mellor et al. 2021): from the forward pass alone (dropout off), the binary code of every ReLU20 unit --
+  the block convs' and every non-`zero` node op's, m = (0 < z <= 20), the indicator of the unit's LINEAR region, a
+  deliberate choice over the classic z > 0, which counts saturated units as active -- gives the kernel matrix
+  K[i, j] = number of units, over the frames valid for both utterances, on which utterances i and j have the same code;
+  score log|det K| (fp64 slogdet on the host; -inf when K is singular, e.g. for a batch with a duplicated utterance).
+  Valid frames of block k: min(T_k, ceil(audio_len / 2^s_k)), s = (0, 0, 1, 2).  K comes from the gate-bit masks a
+  grad plan's forward pass already writes (nbasr_gate_gram, exact integer counts); with grad_norm / snip it reuses
+  their forward pass.
 
 Scored tensors are the ``.weight`` of every Conv1d and Linear (time-reduction and grouped convs, linear edges, classifier);
 LSTM, LayerNorm and biases are not scored ("conv and linear layers", as in the pruning-at-init library).  Per-tensor sums
@@ -22,11 +30,13 @@ import torch
 import torch.nn as nn
 
 from . import _lib
-from .model import ASRModel, FEATURES
+from .model import ASRModel, FEATURES, TR_STRIDES
 from .trainer import ctc_loss_cuda
 
-MEASURES = ('grad_norm', 'snip', 'synflow', 'jacob_cov')
+MEASURES = ('grad_norm', 'snip', 'synflow', 'jacob_cov', 'nwot')
 SEG_CHUNK = 16384          # chunk of nbasr_param_stats (optim.cu)
+# s_k of block k: its frames are the input's halved s_k times, (0, 0, 1, 2)
+LEN_SHIFT = tuple(sum(1 for s in TR_STRIDES[:k + 1] if s == 2) for k in range(len(TR_STRIDES)))
 
 
 def parse_measures(text):
@@ -103,6 +113,50 @@ def jacob_correlation(model, audio):
     return corrcoef_from_gram(G, s, FEATURES * T)
 
 
+def gate_frames(audio_len, T_k, s_k):
+    """Valid frames of a block with T_k frames and length shift s_k: min(T_k, ceil(audio_len / 2^s_k))."""
+    return min(T_k, -(-int(audio_len) >> s_k))
+
+
+def _gate_table(eng, pl):
+    """The plan's ReLU layers as a device array of nbasr_gate_layer, built on first use and kept on the plan."""
+    if getattr(pl, 'gate_table', None) is None:
+        arr = (_lib.GateLayer * len(pl.gates))()
+        for e, (mask, geo, k) in zip(arr, pl.gates):
+            e.mask, e.mask_rows, e.w, e.C = mask.t.data_ptr(), geo.rows, mask.w, geo.C
+            e.Tp, e.T, e.s = geo.Tp, geo.T, LEN_SHIFT[k]
+        pl.gate_table = torch.frombuffer(bytearray(arr), dtype=torch.uint8).to(eng.device)
+    return pl.gate_table
+
+
+def _gate_gram(eng, pl, audio_len):
+    """K (B, B) uint64 numpy from the gate masks of a grad plan's last forward pass; audio_len int64 on the device."""
+    table = _gate_table(eng, pl)
+    B = pl.B
+    K = torch.empty(B, B, dtype=torch.int64, device=eng.device)
+    work = torch.empty(int(eng.lib.nbasr_gate_gram_work_elems(B)), dtype=torch.int64, device=eng.device)
+    _lib.check(eng.lib.nbasr_gate_gram(table.data_ptr(), len(pl.gates), audio_len.data_ptr(), B, K.data_ptr(), work.data_ptr(),
+                                       torch.cuda.current_stream().cuda_stream), 'gate_gram')
+    return K.cpu().numpy().view(np.uint64)
+
+
+def nwot_kernel(model, batch):
+    """NASWOT kernel matrix K (B, B) uint64 of `model` on batch ((audio, audio_len), ...): one forward pass of a grad
+    plan, dropout off, no backward."""
+    eng = model.engine
+    eng.bind()
+    (audio, audio_len) = batch[0]
+    with torch.cuda.device(eng.device):
+        alen = audio_len.to(eng.device, torch.int64).contiguous()
+        pl = eng.forward(audio.to(eng.device, torch.float32).contiguous(), training=False, grad=True)
+        return _gate_gram(eng, pl, alen)
+
+
+def nwot_score(K):
+    """log|det K| in fp64 (numpy.linalg.slogdet); -inf when K is singular."""
+    return float(np.linalg.slogdet(np.asarray(K, dtype=np.float64))[1])
+
+
 def _norm_free_fp32_copy(model):
     """The parameters of model.get_prunable_copy(bn=False) on the fp32 engine.  The module tree is built on the meta device
     and takes the model's tensors (the engine copies them into its own flat buffer when it binds): no host-side default
@@ -145,7 +199,7 @@ def compute_proxies(model, batch, measures=MEASURES, per_layer=False):
     """Zero-cost proxies of `model` on one batch ((audio (B,80,T), audio_len), (targets, targets_len)).
 
     Returns {measure: float}, or with per_layer=True {measure: {parameter name: float}} for grad_norm / snip / synflow
-    (jacob_cov is a whole-network score and stays a float)."""
+    (jacob_cov and nwot are whole-network scores and stay floats)."""
     measures = tuple(measures)
     bad = [m for m in measures if m not in MEASURES]
     if bad:
@@ -158,6 +212,7 @@ def compute_proxies(model, batch, measures=MEASURES, per_layer=False):
     with torch.cuda.device(dev):
         audio = audio.to(dev, torch.float32).contiguous()
         saved_g = eng.flat_g.clone()
+        pl = None
         try:
             if 'grad_norm' in measures or 'snip' in measures:
                 pl = eng.forward(audio, training=False, grad=True)
@@ -172,6 +227,12 @@ def compute_proxies(model, batch, measures=MEASURES, per_layer=False):
                     out['snip'] = {n: v[1] for n, v in st.items()}
             if 'jacob_cov' in measures:
                 out['jacob_cov'] = jacob_cov_score(jacob_correlation(model, audio))
+            if 'nwot' in measures:
+                # the backward pass only reads the gate masks: grad_norm / snip's forward pass is reused as it stands
+                alen = audio_len.to(dev, torch.int64).contiguous()
+                if pl is None:
+                    pl = eng.forward(audio, training=False, grad=True)
+                out['nwot'] = nwot_score(_gate_gram(eng, pl, alen))
         finally:
             eng.flat_g.copy_(saved_g)
         if 'synflow' in measures:

@@ -90,7 +90,7 @@ def build_parser():
     ap.add_argument('--out-pickle', default=None, help='nb-asr style table: header, then rows')
     ap.add_argument('--all', action='store_true', help='evaluate every arch_vec, not one per isomorphism class')
     ap.add_argument('--proxies', type=proxy_list, default=(),
-                    help='comma-separated zero-cost proxies to add as columns: grad_norm,snip,synflow,jacob_cov')
+                    help='comma-separated zero-cost proxies to add as columns: grad_norm,snip,synflow,jacob_cov,nwot')
     ap.add_argument('--proxy-batches', type=int, default=1,
                     help='the proxies are averaged over the first N batches of the evaluation set')
     return ap

@@ -3,8 +3,9 @@
     python tools/bench_proxies.py [--reps 5] [--sample 24] [--out profiles/proxies.json]
 
 * ms per measure (grad_norm and snip share one forward + backward and are timed together) for four archs at B x T = 64 x 500;
+  nwot alone (one forward pass + nbasr_gate_gram) and grad_norm + snip + nwot (nwot reuses their forward pass);
 * the sweep's candidates per second on a fixed sample of unique archs (every k-th of the 8 242), evaluated exactly as
-  nb_asr_b200.sweep does, with and without all four proxies (--proxy-batches 1);
+  nb_asr_b200.sweep does, without proxies, with --proxies nwot and with all five proxies (--proxy-batches 1);
 * the GPU's name and power limit, read in the same run.
 """
 import argparse
@@ -22,7 +23,8 @@ from nb_asr_b200 import data, graph_utils, proxies, sweep  # noqa: E402
 
 ARCHS = {'default': [[1, 0], [1, 0, 0], [1, 0, 0, 0]], 'linear_skips': [[0, 1], [0, 1, 1], [0, 1, 1, 1]],
          'c7d2_skips': [[4, 1], [4, 1, 1], [4, 1, 1, 1]], 'zero_mix': [[5, 1], [1, 1, 0], [5, 0, 1, 1]]}
-GROUPS = {'grad_norm+snip': ('grad_norm', 'snip'), 'jacob_cov': ('jacob_cov',), 'synflow': ('synflow',)}
+GROUPS = {'grad_norm+snip': ('grad_norm', 'snip'), 'jacob_cov': ('jacob_cov',), 'synflow': ('synflow',), 'nwot': ('nwot',),
+          'grad_norm+snip+nwot': ('grad_norm', 'snip', 'nwot')}
 
 
 def gpu_info():
@@ -47,12 +49,25 @@ def time_measures(arch, precision, reps, B=64, T=500):
         torch.cuda.synchronize()
         res[g] = (time.perf_counter() - t0) / reps * 1e3
         res.update({f'value_{k}': v for k, v in vals.items()})
+    # nbasr_gate_gram alone, on the masks of the forward pass nwot just ran (CUDA events)
+    eng = model.engine
+    pl = eng.plan(B, T, False, True)
+    alen = b[0][1].to(torch.int64).contiguous()
+    proxies._gate_gram(eng, pl, alen)
+    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    e0.record()
+    for _ in range(reps):
+        proxies._gate_gram(eng, pl, alen)
+    e1.record()
+    torch.cuda.synchronize()
+    res['gate_gram_call'] = e0.elapsed_time(e1) / reps
+    res['relu_layers'] = len(pl.gates)
     model._engine = None
     return res
 
 
-def sweep_rate(archs, batches, use_proxies):
-    kw = dict(proxies=proxies.MEASURES, proxy_batches=1) if use_proxies else {}
+def sweep_rate(archs, batches, measures):
+    kw = dict(proxies=measures, proxy_batches=1) if measures else {}
     n_ref = sum(int(tl.sum()) for _, (t, tl) in batches)
     sweep.evaluate_arch(archs[0], batches, 0, 'bf16', init='device', conv_gain=101 ** 0.5, n_ref=n_ref, **kw)   # warm-up
     torch.cuda.synchronize()
@@ -81,11 +96,13 @@ def main():
     archs = uniq[::step][:args.sample]
     batches = data.timit_shaped_eval_set(n_utt=1344, batch_size=64, seed=0)
     batches = [((a.cuda(), al.cuda()), (t.cuda(), tl.cuda())) for (a, al), (t, tl) in batches]
-    r0, _ = sweep_rate(archs, batches, False)
-    r1, rows = sweep_rate(archs, batches, True)
-    finite = sum(all(r[m] == r[m] and abs(r[m]) != float('inf') for m in proxies.MEASURES) for r in rows)
-    out['sweep'] = dict(n_archs=len(archs), sample_step=step, archs_per_s=r0, archs_per_s_with_proxies=r1,
-                        rows_with_finite_proxies=finite, eval_batches=len(batches), proxy_batches=1)
+    r0, _ = sweep_rate(archs, batches, ())
+    rn, _ = sweep_rate(archs, batches, ('nwot',))
+    r1, rows = sweep_rate(archs, batches, proxies.MEASURES)
+    finite = {m: sum(r[m] == r[m] and abs(r[m]) != float('inf') for r in rows) for m in proxies.MEASURES}
+    out['sweep'] = dict(n_archs=len(archs), sample_step=step, archs_per_s=r0, archs_per_s_with_nwot=rn,
+                        archs_per_s_with_proxies=r1, measures=list(proxies.MEASURES), rows_with_finite=finite,
+                        eval_batches=len(batches), proxy_batches=1)
     print(json.dumps(out['sweep']), flush=True)
     print(json.dumps(dict(gpu=out['gpu'])))
     if args.out:
