@@ -165,6 +165,11 @@ int64_t nbasr_gconv_mma_pack_elems(int C, int cpg, int ktaps);
  * (dbias may be NULL). BF16 -> tcgen05 kernel, F32 -> SIMT. */
 int nbasr_gconv_wgrad(int dtype, const void* dz, const void* x, int B, int T, int Tp, int C, int cpg,
                       int ktaps, int off0, int dstep, float* dw, float* dbias, void* stream);
+/* The same with X in its own format, multiplied by x_scale as it is read: the scaled fp16 forward activations (S*x, nbasr.h
+ * "scaled fp16") with x_scale = 1/S, so that a 16-bit plan needs no bf16 copy of them.  dz_dtype BF16 takes x_dtype BF16 or
+ * F16; F32 takes F32.  nbasr_gconv_wgrad(dtype, ...) is nbasr_gconv_wgrad_x(dtype, dz, x, dtype, 1, ...). */
+int nbasr_gconv_wgrad_x(int dz_dtype, const void* dz, const void* x, int x_dtype, float x_scale, int B, int T, int Tp, int C,
+                        int cpg, int ktaps, int off0, int dstep, float* dw, float* dbias, void* stream);
 
 /* Element-wise pass through the epilogue: v = src ? src[rho,n] : 0 over rows (b,t) of a padded
  * (B,Tp,C) geometry.  Used for `zero` main ops (ops.py:62-68), the LSTM input dropout

@@ -54,6 +54,7 @@ _SIGS = {
     'nbasr_pack_gconv_mma': [_vp, _vp, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _vp],
     'nbasr_gconv_mma_pack_elems': [C.c_int, C.c_int, C.c_int],
     'nbasr_gconv_wgrad': [C.c_int, _vp, _vp] + [C.c_int] * 8 + [_vp, _vp, _vp],
+    'nbasr_gconv_wgrad_x': [C.c_int, _vp, _vp, C.c_int, _f32] + [C.c_int] * 8 + [_vp, _vp, _vp],
     'nbasr_eltwise': [C.c_int, _vp, _i64, C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(Epilogue), _vp],
     'nbasr_colsum': [C.c_int, _vp, C.c_int, C.c_int, C.c_int, C.c_int, _vp, _vp],
     'nbasr_layernorm_fwd': [C.c_int, _vp, _vp, C.c_int, C.c_int, C.c_int, C.c_int, _vp, _vp, _f32, _vp, _vp, _f32, _vp, _vp],

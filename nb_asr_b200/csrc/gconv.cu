@@ -113,9 +113,10 @@ __global__ void __launch_bounds__(G_NT) gconv_fwd_kernel(nbasr_gconv p) {
 constexpr int W_PAIRS = 7;  // (co,i) pairs per thread: slab pairs <= 160*10 = 1600 <= 7*256
 constexpr int W_FB = 8;
 
-template <typename T>
-__global__ void __launch_bounds__(G_NT) gconv_wgrad_kernel(const T* __restrict__ dz, const T* __restrict__ x, int B,
-                                                           int Tt, int Tp, int C, int cpg, int ktaps, int off0,
+// X is staged as x * x_scale (x_scale = 1/S for the forward's scaled fp16 activations)
+template <typename TD, typename TX>
+__global__ void __launch_bounds__(G_NT) gconv_wgrad_kernel(const TD* __restrict__ dz, const TX* __restrict__ x, float x_scale,
+                                                           int B, int Tt, int Tp, int C, int cpg, int ktaps, int off0,
                                                            int dstep, float* __restrict__ dw) {
   extern __shared__ float smem[];
   const int CS = slab_channels(cpg);
@@ -145,7 +146,7 @@ __global__ void __launch_bounds__(G_NT) gconv_wgrad_kernel(const T* __restrict__
         for (int i = 0; i < 8; ++i) v[i] = 0.f;
       }
 #pragma unroll
-      for (int i = 0; i < 8; ++i) xs[r * CS + g8 * 8 + i] = v[i];
+      for (int i = 0; i < 8; ++i) xs[r * CS + g8 * 8 + i] = v[i] * x_scale;
     }
     for (int idx = tid; idx < G_TT * vec; idx += G_NT) {
       int r = idx / vec, g8 = idx % vec;
@@ -266,28 +267,34 @@ int nbasr_pack_gconv_dgrad(const float* w, float* wt, int C, int cpg, int ktaps,
   return 0;
 }
 
-int nbasr_gconv_wgrad(int dtype, const void* dz, const void* x, int B, int T, int Tp, int C, int cpg, int ktaps,
-                      int off0, int dstep, float* dw, float* dbias, void* stream) {
+int nbasr_gconv_wgrad_x(int dz_dtype, const void* dz, const void* x, int x_dtype, float x_scale, int B, int T, int Tp, int C,
+                        int cpg, int ktaps, int off0, int dstep, float* dw, float* dbias, void* stream) {
   NBASR_REQUIRE(cpg == 6 || cpg == 8 || cpg == 10 || cpg == 12, "cpg");
   NBASR_REQUIRE(ktaps <= 7 && (dstep == 1 || dstep == 2), "taps");
+  NBASR_REQUIRE(dz_dtype == NBASR_BF16 ? (x_dtype == NBASR_BF16 || x_dtype == NBASR_F16) : (dz_dtype == NBASR_F32 && x_dtype == NBASR_F32),
+                "dtypes: bf16 dz with bf16 / fp16 x, or fp32 dz and x");
   if (B <= 0 || T <= 0) return 0;
-  if (dtype == NBASR_BF16 && !nbasr_env_flag(NBASR_ENV_FORCE_SIMT))
-    return sm100_gconv_wgrad(dz, x, B, T, Tp, C, cpg, ktaps, off0, dstep, dw, dbias, as_stream(stream));
-  if (dbias && nbasr_colsum(dtype, dz, B, T, Tp, C, dbias, stream)) return 1;
+  if (dz_dtype == NBASR_BF16 && !nbasr_env_flag(NBASR_ENV_FORCE_SIMT))
+    return sm100_gconv_wgrad(dz, x, x_dtype == NBASR_F16, x_scale, B, T, Tp, C, cpg, ktaps, off0, dstep, dw, dbias, as_stream(stream));
+  if (dbias && nbasr_colsum(dz_dtype, dz, B, T, Tp, C, dbias, stream)) return 1;
   int CS = slab_channels(cpg);
   dim3 grid((C + CS - 1) / CS, B);
   size_t sm = wgrad_smem(cpg);
-  if (dtype == NBASR_BF16) {
-    static DevOnce attr;
-    if (!attr) { cudaFuncSetAttribute(gconv_wgrad_kernel<bf16>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024); attr = true; }
-    gconv_wgrad_kernel<bf16><<<grid, G_NT, sm, as_stream(stream)>>>((const bf16*)dz, (const bf16*)x, B, T, Tp, C, cpg, ktaps, off0, dstep, dw);
-  } else {
-    static DevOnce attr;
-    if (!attr) { cudaFuncSetAttribute(gconv_wgrad_kernel<float>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024); attr = true; }
-    gconv_wgrad_kernel<float><<<grid, G_NT, sm, as_stream(stream)>>>((const float*)dz, (const float*)x, B, T, Tp, C, cpg, ktaps, off0, dstep, dw);
-  }
+  auto launch = [&](auto kern, auto dzp, auto xp) {
+    static DevOnce attr;     // one latch per kernel instantiation (the lambda is instantiated per argument types)
+    if (!attr) { cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024); attr = true; }
+    kern<<<grid, G_NT, sm, as_stream(stream)>>>(dzp, xp, x_scale, B, T, Tp, C, cpg, ktaps, off0, dstep, dw);
+  };
+  if (dz_dtype == NBASR_F32) launch(gconv_wgrad_kernel<float, float>, (const float*)dz, (const float*)x);
+  else if (x_dtype == NBASR_F16) launch(gconv_wgrad_kernel<bf16, f16>, (const bf16*)dz, (const f16*)x);
+  else launch(gconv_wgrad_kernel<bf16, bf16>, (const bf16*)dz, (const bf16*)x);
   NBASR_CHECK_LAUNCH();
   return 0;
+}
+
+int nbasr_gconv_wgrad(int dtype, const void* dz, const void* x, int B, int T, int Tp, int C, int cpg, int ktaps,
+                      int off0, int dstep, float* dw, float* dbias, void* stream) {
+  return nbasr_gconv_wgrad_x(dtype, dz, x, dtype, 1.f, B, T, Tp, C, cpg, ktaps, off0, dstep, dw, dbias, stream);
 }
 
 }  // extern "C"

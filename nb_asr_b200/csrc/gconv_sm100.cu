@@ -20,8 +20,9 @@
 //    are the reduction index).  ALL taps share one M=128 x N=64*ceil(k/2) MMA per 16-frame K step: the A
 //    descriptor's "leading byte offset" makes rows 64..127 the same dZ tile shifted by `dstep` frames, the
 //    B descriptor's makes N atom i the same X tile shifted by 2 i dstep frames, so (atom i, rows 64-127)
-//    gives tap 2i and (atom i, rows 0-63) tap 2i+1.  Diagonal blocks are extracted from TMEM and atomically
-//    added to the fp32 gradient.
+//    gives tap 2i and (atom i, rows 0-63) tap 2i+1.  Diagonal blocks are extracted from TMEM, assembled into the slab's
+//    contiguous gradient run in shared memory and added to the fp32 gradient with 16-byte reductions.  X may be the forward's scaled fp16 activation: the drain warps convert each landed tile
+//    to bf16 in place before the MMAs read it, so a 16-bit plan keeps no bf16 copy of it.
 #include <cuda.h>
 
 #include "common.cuh"
@@ -306,6 +307,8 @@ constexpr int WG_SMEM = NSTAGE * WG_STAGE + 1024 + 256;
 struct GcWgArgs {
   int B, T, C, cpg, OUT, ktaps, dstep, off0;
   int nslabs, nchunks, nunits, nlanes, dbg;
+  int x_f16;      // X is fp16 holding x / x_scale (the forward's scaled activation): converted to bf16 in shared memory
+  float x_scale;
   float* dw;
   float* dbias;   // optional: db[c] += sum_t dZ[t][c], computed by the tensor core against a column of ones
 };
@@ -319,9 +322,9 @@ gconv_mma_wgrad_kernel(const __grid_constant__ CUtensorMap tmDZ, const __grid_co
   auto full_bar = [&](int s) { return bar0 + 8u * s; };
   auto empty_bar = [&](int s) { return bar0 + 8u * (NSTAGE + s); };
   const uint32_t tfull = bar0 + 8u * (2 * NSTAGE);
-  auto ready_bar = [&](int s) { return bar0 + 8u * (2 * NSTAGE + 1 + s); };     // "ones column written" (bias gradient)
+  auto ready_bar = [&](int s) { return bar0 + 8u * (2 * NSTAGE + 1 + s); };     // X tile converted / ones column written
   uint32_t* tptr = reinterpret_cast<uint32_t*>(al + NSTAGE * WG_STAGE + 8 * (3 * NSTAGE + 2));
-  // warp roles: 0..3 drain (warp 0 also plants the ones column), 4 producer, 5 MMA issue (highest id: issue priority)
+  // warp roles: 0..3 drain (and, in the main loop, X tile preparation), 4 producer, 5 MMA issue (highest id: issue priority)
   const int warp = uniform_warp_idx(), lane = threadIdx.x & 31;
   const int slab = blockIdx.x % p.nslabs;
   const int lane_id = blockIdx.x / p.nslabs;
@@ -332,7 +335,7 @@ gconv_mma_wgrad_kernel(const __grid_constant__ CUtensorMap tmDZ, const __grid_co
   if (warp == 4 && lane == 0) {
     prefetch_tmap(&tmDZ);
     prefetch_tmap(&tmX);
-    for (int s = 0; s < NSTAGE; ++s) { mbar_init(full_bar(s), 1); mbar_init(empty_bar(s), 1); mbar_init(ready_bar(s), 1); }
+    for (int s = 0; s < NSTAGE; ++s) { mbar_init(full_bar(s), 1); mbar_init(empty_bar(s), 1); mbar_init(ready_bar(s), 4); }
     mbar_init(tfull, 1);
     fence_barrier_init();
   }
@@ -371,8 +374,8 @@ gconv_mma_wgrad_kernel(const __grid_constant__ CUtensorMap tmDZ, const __grid_co
       uint32_t phase = 0;
       bool first = true;
       for (int u = lane_id; u < p.nunits; u += p.nlanes) {
-        // with a bias gradient the stage is usable once the helper warp has planted the ones column (below)
-        mbar_wait(p.dbias ? ready_bar(stage) : full_bar(stage), phase);
+        // with fp16 X or a bias gradient the stage is usable once the drain warps have prepared its X tile (below)
+        mbar_wait((p.x_f16 || p.dbias) ? ready_bar(stage) : full_bar(stage), phase);
         const uint32_t sa = base + stage * WG_STAGE;
         tcgen05_fence_after();
         const uint64_t ad0 = make_smem_desc(sa, (uint32_t)p.dstep * 128u, 1024);
@@ -391,18 +394,40 @@ gconv_mma_wgrad_kernel(const __grid_constant__ CUtensorMap tmDZ, const __grid_co
       __syncwarp();
     }
   } else if (has_work) {
-    if (warp == 0 && p.dbias) {
-      // Bias gradient = dZ^T 1: channel 63 of the X window (never part of a slab) <- 1.0 for every frame row (element 7 of
-      // the 16-byte chunk 7, at its 128B-swizzled position chunk ^ (row & 7)).  Done by this otherwise idle epilogue warp as
-      // soon as a stage has landed, OFF the MMA warp's critical path (ncu r2: tensor pipe 37 % busy with the write + proxy
-      // fence in front of every unit's MMAs).
+    if (p.x_f16 || p.dbias) {
+      // Warps 0..3, idle until the drain, prepare each landed X tile for the MMAs, each on its own AROWS / 4 rows, OFF the MMA
+      // warp's critical path (ncu r2: tensor pipe 37 % busy with the ones-column write + proxy fence in front of every unit's
+      // MMAs when the MMA warp did it itself):
+      //  * fp16 X -> bf16 in place, x * x_scale rounded once (x_scale = 1/S is a power of two: exact before the rounding).
+      //    Element-wise, so the 128B swizzle (a permutation of whole 16-byte chunks within a row) does not matter.
+      //  * bias gradient = dZ^T 1: channel 63 of the X window (never part of a slab) <- 1.0 for every frame row (element 7 of
+      //    the 16-byte chunk 7, at its swizzled position chunk ^ (row & 7)).
+      constexpr int QROWS = AROWS / 4;
+      const int r0 = warp * QROWS;
       int stage = 0;
       uint32_t phase = 0;
       for (int u = lane_id; u < p.nunits; u += p.nlanes) {
         mbar_wait(full_bar(stage), phase);
         uint8_t* xb = al + stage * WG_STAGE + DZ_BYTES;
-        for (int r = lane; r < AROWS; r += 32)
-          *reinterpret_cast<uint16_t*>(xb + r * 128 + ((7 ^ (r & 7)) << 4) + 14) = 0x3F80;
+        if (p.x_f16) {
+#pragma unroll 3
+          for (int i = lane; i < QROWS * 8; i += 32) {          // 16-byte chunks, 8 per row: 9 per lane
+            const int r = r0 + (i >> 3), ch = i & 7;
+            uint4* cp = reinterpret_cast<uint4*>(xb + r * 128 + ch * 16);
+            uint4 w = *cp;
+            uint32_t* h = &w.x;
+#pragma unroll
+            for (int e = 0; e < 4; ++e) {
+              const float2 f = f16x2_to_f2(h[e]);
+              h[e] = f2_to_bf16x2(f.x * p.x_scale, f.y * p.x_scale);
+            }
+            if (p.dbias && ch == (7 ^ (r & 7))) w.w = (w.w & 0xffffu) | (0x3F80u << 16);
+            *cp = w;
+          }
+        } else {
+          for (int r = r0 + lane; r < r0 + QROWS; r += 32)
+            *reinterpret_cast<uint16_t*>(xb + r * 128 + ((7 ^ (r & 7)) << 4) + 14) = 0x3F80;
+        }
         asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
         __syncwarp();
         if (lane == 0) mbar_arrive(ready_bar(stage));
@@ -415,6 +440,16 @@ gconv_mma_wgrad_kernel(const __grid_constant__ CUtensorMap tmDZ, const __grid_co
     const int co = cbox + co_l;
     const bool row_ok = co_l >= coff && co_l < coff + p.OUT && co < p.C;
     const int g_l = (co_l - coff) / p.cpg;
+    // The slab's gradient dw[c0 .. c0 + nco)[cpg][ktaps] is ONE contiguous run of nco * cpg * ktaps floats (<= 16 KB).  The
+    // drain warps assemble it in the stage buffers, idle once every MMA has completed (tfull) -- each element is written
+    // exactly once: a thread owns one output channel, the two TMEM halves hold disjoint taps -- and add it to global memory
+    // with 16-byte reductions, 4x fewer than one fp32 atomic per element (those were ~15 % of the kernel's time).  The run
+    // starts `pad` floats into shared memory so that its 16-byte-aligned global stretch is 16-byte aligned there too.
+    const int nco = min(p.OUT, p.C - c0);
+    const int nrun = nco * p.cpg * p.ktaps;
+    float* g = p.dw + (int64_t)c0 * p.cpg * p.ktaps;
+    const int head = min(nrun, (int)(((16u - (uint32_t)(reinterpret_cast<uintptr_t>(g) & 15u)) & 15u) >> 2));
+    float* run = reinterpret_cast<float*>(al) + ((4 - head) & 3);
     mbar_wait(tfull, 0);
     tcgen05_fence_after();
     for (int pr = 0; pr < npairs; ++pr) {
@@ -425,14 +460,23 @@ gconv_mma_wgrad_kernel(const __grid_constant__ CUtensorMap tmDZ, const __grid_co
       const int tap = half ? 2 * pr : 2 * pr + 1;
       // column 63 of atom 0, rows 64..127 (tap 0, unshifted dZ) = sum_t dZ[t][co]
       if (pr == 0 && p.dbias && row_ok && half) atomicAdd(p.dbias + co, v[63]);
-      if (row_ok && tap < p.ktaps && !(p.dbg & 1024)) {
-        float* dst = p.dw + ((int64_t)co * p.cpg) * p.ktaps + tap;
+      if (row_ok && tap < p.ktaps) {
+        float* dst = run + (co_l - coff) * p.cpg * p.ktaps + tap;
 #pragma unroll
         for (int i = 0; i < 64; ++i) {
           const int il = i - coff - g_l * p.cpg;
-          if (il >= 0 && il < p.cpg) atomicAdd(dst + il * p.ktaps, v[i]);
+          if (il >= 0 && il < p.cpg) dst[il * p.ktaps] = v[i];
         }
       }
+    }
+    named_bar_sync(1, 128);
+    if (!(p.dbg & 1024)) {
+      const int tid = threadIdx.x;                    // 0 .. 127: the drain warps
+      const int nvec = (nrun - head) >> 2, tail = head + 4 * nvec;
+      if (tid < head) atomicAdd(g + tid, run[tid]);
+      for (int j = tid; j < nvec; j += 128)
+        atomicAdd(reinterpret_cast<float4*>(g + head) + j, reinterpret_cast<const float4*>(run + head)[j]);
+      if (tail + tid < nrun) atomicAdd(g + tail + tid, run[tail + tid]);
     }
   }
   tcgen05_fence_before();
@@ -514,9 +558,11 @@ int sm100_gconv_fwd(const nbasr_gconv* g, cudaStream_t st) {
   return 0;
 }
 
-int sm100_gconv_wgrad(const void* dz, const void* x, int B, int T, int Tp, int C, int cpg, int ktaps, int off0, int dstep,
-                      float* dw, float* dbias, cudaStream_t st) {
+int sm100_gconv_wgrad(const void* dz, const void* x, int x_f16, float x_scale, int B, int T, int Tp, int C, int cpg, int ktaps,
+                      int off0, int dstep, float* dw, float* dbias, cudaStream_t st) {
   GcWgArgs a{};
+  a.x_f16 = x_f16;
+  a.x_scale = x_scale;
   a.B = B; a.T = T; a.C = C; a.cpg = cpg; a.OUT = wg_slab_out(cpg); a.ktaps = ktaps; a.dstep = dstep; a.off0 = off0;
   NBASR_REQUIRE(off0 >= -NBASR_PAD_L && (ktaps - 1) * dstep <= AROWS - GT && dstep <= DZROWS - GT, "tap reach");
   a.nslabs = (C + a.OUT - 1) / a.OUT;

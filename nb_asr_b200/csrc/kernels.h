@@ -80,8 +80,9 @@ int sm100_gconv_fwd(const nbasr_gconv* p, cudaStream_t st);
 // several chained grouped-conv edges in one launch (gconv_chain_sm100.cu)
 int sm100_gconv_chain(const nbasr_gconv* nodes, int n, int fused, void* work, int64_t work_bytes, cudaStream_t st);
 int64_t sm100_gconv_chain_work_bytes(int B, int T, int C, int cpg, int n);
-int sm100_gconv_wgrad(const void* dz, const void* x, int B, int T, int Tp, int C, int cpg, int ktaps, int off0, int dstep,
-                      float* dw, float* dbias, cudaStream_t st);
+// x_f16: x is fp16 holding x / x_scale, converted to bf16 in shared memory (otherwise bf16, x_scale unused)
+int sm100_gconv_wgrad(const void* dz, const void* x, int x_f16, float x_scale, int B, int T, int Tp, int C, int cpg, int ktaps,
+                      int off0, int dstep, float* dw, float* dbias, cudaStream_t st);
 
 // cluster / tcgen05 LSTM recurrence (lstm_sm100.cu)
 int sm100_lstm_fwd(const float* gx, const void* w_packed, int T, int B, int H, void* h_seq, int h_dtype, int64_t h_bs, int64_t h_rs,

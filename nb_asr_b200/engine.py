@@ -36,6 +36,28 @@ def _ptr(t, off_elems=0):
     return t.data_ptr() + off_elems * t.element_size()
 
 
+def dense_wgrad_inputs(arch, use_norm, use_rnn, input_dropout=False):
+    """Names of the forward activations that a dense (GEMM) weight gradient reads: the input of each block's time-reduction
+    conv, of every `linear` edge and of the LSTM input projection (the encoder output, or its input-dropout copy).  In a
+    16-bit grad plan exactly these get an unscaled bf16 twin: one tcgen05.mma cannot take the fp16 activation and the bf16
+    gradient together.  The grouped-conv weight gradient needs none; it converts the fp16 tile itself (nbasr_gconv_wgrad_x).
+    Names: 'input' (the transposed features), 'b{i}.ln' (block i's LayerNorm), 'b{i}.c{c}.n{n}' (node n of cell c),
+    'b{i}.c{c}.ln' (cell c's LayerNorm) and 'lstm_in' (the LSTM's input dropout, only in plans with dropout)."""
+    ops = [nd[0] for nd in arch]
+    names = {'input'}
+    for i, ncells in enumerate(CELLS_PER_BLOCK):
+        cin = f'b{i}.ln'
+        for c in range(ncells):
+            outs = [cin] + [f'b{i}.c{c}.n{n}' for n in range(len(ops))]       # node n reads outs[n]
+            names.update(outs[n] for n, op in enumerate(ops) if op == 'linear')
+            cin = f'b{i}.c{c}.ln' if use_norm else outs[-1]
+        if i < len(CELLS_PER_BLOCK) - 1:
+            names.add(cin)
+        elif use_rnn:
+            names.add('lstm_in' if input_dropout else cin)
+    return names
+
+
 class _Geo:
     """Padded channels-last geometry of one encoder block: (B, Tp, C), frame t at row b*Tp+PAD_L+t."""
 
@@ -448,9 +470,9 @@ class Engine:
     def plan(self, B, T, training, grad=None, input_grad=False):
         """Plans are cached per (B, T, training, grad[, 'input_grad']), least recently used first.  `training` switches
         dropout on; `grad` (default: training) says whether a backward pass may follow: only then are gate-bit masks, bf16
-        twins of the forward activations and the backward call list built (an eval step needs none of them).  `input_grad`
+        twins of the forward activations a dense weight gradient reads and the backward call list built (an eval step needs none of them).  `input_grad`
         (implies grad) appends the gradient wrt the input features to the backward pass: pl.daudio (B, 80, T) fp32.  A plan
-        owns every activation / mask / gradient buffer of its shape (about 3.7 GB at 64 x 500) plus the CUDA graphs and CTC workspaces captured on it, so
+        owns every activation / mask / gradient buffer of its shape (at 64 x 500 on the default arch: 4.6 GB for a grad plan, 3.0 GB for an eval plan) plus the CUDA graphs and CTC workspaces captured on it, so
         loaders whose padded length changes from batch to batch would otherwise grow without bound: beyond `max_plans`
         (NBASR_MAX_PLANS, default 6) the oldest plan is dropped and its memory returns to the allocator."""
         grad = bool(training) if grad is None else bool(grad)
@@ -469,9 +491,11 @@ class Engine:
         return pl
 
     def _plan_bytes_estimate(self, B, T, grad):
-        """Rough size of a plan's arena: per encoder block (2 + 4 per cell) activation buffers, with gradients also their
-        bf16 twins, 7 gradient buffers and 1 bit per element of gate masks; head and small buffers on top."""
+        """Rough size of a plan's arena: per encoder block (2 + 4 per cell) activation buffers, with gradients also the
+        bf16 twins of those a dense weight gradient reads, 7 gradient buffers and 1 bit per element of gate masks; head and
+        small buffers on top."""
         es = 2 if self.dt == BF16 else 4
+        twins = dense_wgrad_inputs(self.model.arch_desc, self.model.use_norm, self.model.use_rnn) if self.adt != self.dt else ()
         total, Tcur = B * (T + 16) * FEATURES * es * 2, T
         for i in range(4):
             Tcur = Tcur if TR_STRIDES[i] == 1 else (Tcur + 1) // 2
@@ -480,7 +504,8 @@ class Engine:
             nbuf = 2 + 4 * CELLS_PER_BLOCK[i]
             total += per * nbuf
             if grad:
-                total += per * (nbuf * (1 if self.adt != self.dt else 0) + 7) + per * nbuf // (8 * es) + per // 4
+                ntw = sum(1 for n in twins if n.startswith(f'b{i}.'))
+                total += per * (ntw + 7) + per * nbuf // (8 * es) + per // 4
         total += B * Tcur * (4 * HIDDEN * 4 * (3 if grad else 1) + HP * 2 + HIDDEN * 4 * 3 + 49 * 4 * 3)
         return int(total * 1.05) + (8 << 20)
 
@@ -504,21 +529,25 @@ class Engine:
             return salt[0] * 0x9E3779B1
 
         adt, tadt, S = self.adt, self.tadt, self.S
-        bcopy = {}          # id(forward activation) -> its unscaled bf16 copy (training plans of the 16-bit mode)
+        twin_plan = grad and adt != dt
+        twin_names = dense_wgrad_inputs(m.arch_desc, m.use_norm, m.use_rnn, input_dropout=drop_p > 0) if twin_plan else ()
+        bcopy = {}          # id(forward activation) -> its unscaled bf16 twin (grad plans of the 16-bit mode)
+        pl.twins = {}       # activation name -> bf16 twin
 
         def zbuf(rows, cols, dtype=None):
             return arena.zeros((rows, cols), tdt if dtype is None else dtype)
 
-        def zact(rows, cols, copy=False):
-            """forward activation buffer (activation format) and, if asked for in a 16-bit training plan, its bf16 twin"""
+        def zact(rows, cols, name=None):
+            """forward activation buffer (activation format) and, if a dense weight gradient reads it in a 16-bit grad
+            plan, its bf16 twin"""
             t = arena.zeros((rows, cols), tadt)
-            if copy and grad and adt != dt:
-                bcopy[id(t)] = arena.zeros((rows, cols), tdt)
+            if name in twin_names:
+                bcopy[id(t)] = pl.twins[name] = arena.zeros((rows, cols), tdt)
             return t
 
         def Bc(t):
-            """the tensor a weight gradient reads for forward activation t"""
-            return bcopy.get(id(t), t)
+            """the tensor a dense weight gradient reads for forward activation t"""
+            return bcopy[id(t)] if twin_plan else t
 
         def cptr(t):
             c = bcopy.get(id(t))
@@ -566,7 +595,7 @@ class Engine:
         # ---- input
         pl.audio = arena.zeros((B, FEATURES, T), torch.float32)
         g_in = _Geo(B, T, FEATURES)
-        x_in = zact(g_in.rows, FEATURES, copy=True)
+        x_in = zact(g_in.rows, FEATURES, 'input')
         call(fwd, lib.nbasr_transpose_in, pl.audio.data_ptr(), x_in.data_ptr(), adt, B, FEATURES, T, g_in.Tp, S)
         if cptr(x_in):
             call(fwd, lib.nbasr_transpose_in, pl.audio.data_ptr(), cptr(x_in), dt, B, FEATURES, T, g_in.Tp, 1.0)
@@ -600,8 +629,7 @@ class Engine:
             a_ptr_b = _ptr(Bc(prev), (PAD_L - lpad) * pg.C)      # the same rows of the bf16 copy (weight gradient)
             epi = self._epi(Cc, bias=self.P(cname + '.bias'), relu=1, out=z.data_ptr(), mask_out=zmask, mask_rows=geo.rows, fwd=True)
             gemm(fwd, a_ptr, pg.Tp * pg.C, s * pg.C, B, Ti, K, Cc, wf_ptr, K, PAD_L, Tp, 1, epi, dtype=adt)
-            n_ops = [nd[0] != 'zero' for nd in arch]        # which nodes hold a parametrised op (and read a bf16 copy)
-            y = zact(geo.rows, Cc, copy=True)
+            y = zact(geo.rows, Cc, f'b{i}.ln')
             mean0 = zbuf(geo.rows, 1, torch.float32)
             rstd0 = zbuf(geo.rows, 1, torch.float32)
             lname = self.block_ln[i]
@@ -611,7 +639,7 @@ class Engine:
             rec = dict(i=i, geo=geo, prev=prev, pg=pg, z=z, zmask=zmask, y=y, mean=mean0, rstd=rstd0, cells=[],
                        a_ptr=a_ptr_b, K=K, s=s, lpad=lpad)
             cur = y
-            for cellname in self.block_cells[i]:
+            for ci, cellname in enumerate(self.block_cells[i]):
                 outs = [cur]
                 crec = dict(name=cellname, outs=outs, masks=[], nodes=[])
                 chain = []
@@ -619,9 +647,7 @@ class Engine:
                     op, branches = node[0], node[1:]
                     src = outs[-1]
                     skips = [outs[k] for k, bit in enumerate(branches) if bit]
-                    # node n's output feeds node n+1's op (bf16 copy for its weight gradient); the last node's output feeds
-                    # the cell LayerNorm, or -- without norm -- the next cell / block / LSTM directly
-                    o = zact(geo.rows, Cc, copy=(n_ops[n + 1] if n + 1 < len(arch) else not m.use_norm))
+                    o = zact(geo.rows, Cc, f'b{i}.c{ci}.n{n}')
                     pn = f'{cellname}.nodes.{n}.op'
                     nrec = dict(op=op, branches=list(branches), pn=pn, mask=None, salt=0)
                     adds = [t.data_ptr() for t in skips]
@@ -664,7 +690,7 @@ class Engine:
                     outs.append(o)
                 flush_chain(fwd, chain)
                 if m.use_norm:
-                    co = zact(geo.rows, Cc, copy=True)
+                    co = zact(geo.rows, Cc, f'b{i}.c{ci}.ln')
                     mean = zbuf(geo.rows, 1, torch.float32)
                     rstd = zbuf(geo.rows, 1, torch.float32)
                     call(fwd, lib.nbasr_layernorm_fwd, adt, outs[-1].data_ptr(), co.data_ptr(), B, Ti, Tp, Cc,
@@ -692,7 +718,7 @@ class Engine:
         if m.use_rnn:
             ln = self.lstm_name
             if drop_p > 0:
-                lin = zact(geo3.rows, C3, copy=True)
+                lin = zact(geo3.rows, C3, 'lstm_in')
                 dmask = _Mask(geo3.rows, C3, 32, arena)
                 pl.keep.append(dmask)
                 epi = self._epi(C3, drop_p=drop_p, salt=next_salt(), out=lin.data_ptr(), mask_out=dmask, mask_rows=geo3.rows,
@@ -846,7 +872,7 @@ class Engine:
                     # input-gradient chain first (it produces the dZ of every node), then the chain's weight gradients
                     flush_chain(bwd, chain)
                     for a_ in chain_wg:
-                        call(bwd, lib.nbasr_gconv_wgrad, *a_)
+                        call(bwd, lib.nbasr_gconv_wgrad_x, *a_)
                     del chain_wg[:]
 
                 for j in range(nn_ - 1, -1, -1):
@@ -880,7 +906,8 @@ class Engine:
                     else:
                         d = dzb[j]
                         k, dd, lp = nrec['k'], nrec['d'], nrec['lp']
-                        chain_wg.append((dt, d.data_ptr(), Bc(src).data_ptr(), B, Ti, Tp, Cc, Cc // 100, k, -lp, dd,
+                        # reads the forward activation itself: fp16 S*x in the 16-bit mode, un-scaled while it is staged
+                        chain_wg.append((dt, d.data_ptr(), src.data_ptr(), adt, 1.0 / S, B, Ti, Tp, Cc, Cc // 100, k, -lp, dd,
                                          self.G(pn + '.conv.weight'), self.G(pn + '.conv.bias')))
                         gc = GConv()
                         gc.dtype, gc.x, gc.B, gc.T, gc.Tp, gc.C, gc.cpg = dt, d.data_ptr(), B, Ti, Tp, Cc, Cc // 100

@@ -51,8 +51,8 @@ def op_work(fn_name, args, es):
             fl, by = fl + f1, by + b1
         g = args[0][0]
         return f'gconv C={g.C} chain of {args[1]}', fl, by
-    if fn_name == 'nbasr_gconv_wgrad':
-        dt, dz, x, B, T, Tp, Cc, cpg, k = args[:9]
+    if fn_name in ('nbasr_gconv_wgrad', 'nbasr_gconv_wgrad_x'):
+        B, T, Tp, Cc, cpg, k = args[3:9] if fn_name == 'nbasr_gconv_wgrad' else args[5:11]
         el = B * T * Cc
         return f'gconv_wgrad C={Cc} k={k}', 2.0 * el * cpg * k, el * es * 2
     if fn_name in ('nbasr_layernorm_fwd', 'nbasr_layernorm_bwd'):
