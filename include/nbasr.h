@@ -249,6 +249,27 @@ int nbasr_ctc(const float* logp, int B, int T, int V, const int32_t* targets, in
               const int64_t* audio_len, int len_div, const int64_t* targets_len, float* nll, float* loss,
               float* dlogits, float* work, void* stream);
 
+/* CTC forced alignment: the Viterbi path of the known target sequence through the CTC trellis (where each phone of the
+ * transcript sits in time; what torchaudio.functional.forced_align computes one utterance at a time).  Inputs exactly as
+ * nbasr_ctc: T_b = min(T, audio_len[b] / len_div) frames, S_b = min(S, targets_len[b]) tokens.
+ *   alpha_0(0) = logp[0, 0], alpha_0(1) = logp[0, ext[1]], other states -inf; over the 2S_b + 1 extended states
+ *   alpha_t(s) = max(alpha_{t-1}(s), alpha_{t-1}(s-1), alpha_{t-1}(s-2) [ext[s] != blank, ext[s] != ext[s-2]]) + logp[t, ext[s]]
+ *   (one fp32 add after an exact max).  Ties go to the smaller jump (stay, then s-1, then s-2); at the end the trailing
+ *   blank 2S_b wins over the last label 2S_b - 1 unless the label is strictly better.
+ * Outputs: score[b] = alpha at the chosen end state = max over CTC paths of sum_t logp[t, path_t] (-inf: no path, i.e.
+ * T_b < S_b + adjacent repeats with finite log-probs; 0 for T_b = S_b = 0); labels (B,T) class of each frame on the path
+ * (0 = blank), tok (B,T) index j of the target token the frame emits (-1: blank), start / end (B,S) first frame and one
+ * past the last frame of token j.  Frames t >= T_b, tokens j >= S_b and every output of a row without a path are -1.
+ * A target id outside [1, V) is found on the device: that row gets score NaN and -1 outputs (the call returns 0).
+ * Error (non-zero return): S > 511.  work: nbasr_ctc_align_work_bytes(B, T, S) bytes = 8 * B * T * ceil((2S+1)/32) when
+ * the backpointers (2 bits per frame and state) do not fit in shared memory, i.e. ceil((2S+1)/32) * (T + 32) > 25 600;
+ * 0 otherwise, and work may then be NULL. */
+int nbasr_ctc_align(const float* logp, int B, int T, int V, const int32_t* targets, int S,
+                    const int64_t* audio_len, int len_div, const int64_t* targets_len,
+                    int32_t* labels, int32_t* tok, int32_t* start, int32_t* end, float* score,
+                    void* work, void* stream);
+int64_t nbasr_ctc_align_work_bytes(int B, int T, int S);
+
 /* Greedy CTC decode + fold + Levenshtein PER (trainer.py:229-247 with beam search replaced by
  * argmax/merge-repeats/drop-blank, tf/metrics/ctc.py:76-81; fold encoder.py:64-74 via `lut`
  * (V entries) or NULL).  Outputs: hyp (B,T) int32 folded hypotheses, hyp_len (B), dist (B) edit

@@ -75,6 +75,8 @@ _SIGS = {
                        _vp, _vp, _vp],
     'nbasr_head_bwd_dh': [C.c_int, C.c_int, C.c_int, C.c_int, _vp, _vp, _vp, _i64, _i64, _vp, _vp],
     'nbasr_ctc': [_vp, C.c_int, C.c_int, C.c_int, _vp, C.c_int, _vp, C.c_int, _vp, _vp, _vp, _vp, _vp, _vp],
+    'nbasr_ctc_align': [_vp, C.c_int, C.c_int, C.c_int, _vp, C.c_int, _vp, C.c_int, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp],
+    'nbasr_ctc_align_work_bytes': [C.c_int] * 3,
     'nbasr_greedy_per': [_vp, C.c_int, C.c_int, C.c_int, _vp, C.c_int, _vp, C.c_int, _vp, _vp, _vp, _vp, _vp, _vp,
                          _vp, _vp],
     'nbasr_beam_per': [_vp, C.c_int, C.c_int, C.c_int, _vp, C.c_int, C.c_int, C.c_int, _vp, C.c_int, _vp, _vp, _vp, _vp, _vp, _vp,
@@ -121,6 +123,7 @@ def load():
     lib.nbasr_gconv_chain_work_bytes.restype = C.c_int64
     lib.nbasr_logmel_work_floats.restype = C.c_int64
     lib.nbasr_gate_gram_work_elems.restype = C.c_int64
+    lib.nbasr_ctc_align_work_bytes.restype = C.c_int64
     lib.nbasr_last_error.restype = C.c_char_p
     lib.nbasr_last_error.argtypes = []
     _lib = lib

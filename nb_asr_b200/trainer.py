@@ -101,6 +101,35 @@ def ctc_loss_cuda(logp, output_len_src, len_div, targets, targets_len, dlogits=N
     return ws.loss, ws.nll
 
 
+Alignment = collections.namedtuple('Alignment', 'labels tok start end score')
+Alignment.__doc__ = """CTC forced alignment of a batch (nbasr_ctc_align, include/nbasr.h), device tensors:
+labels (B,T) int32 class of each output frame on the best path (0 = blank), tok (B,T) int32 index of the target token
+the frame emits (-1 on blanks), start / end (B,S) int32 half-open frame span of each target token, score (B,) fp32
+best path log-probability (-inf: the row has no path; NaN: a target id outside [1, V)).  -1 marks frames past the
+output length, tokens past the target length and every output of a row without a path."""
+
+
+def ctc_align_cuda(logp, output_len_src, len_div, targets, targets_len):
+    """Viterbi alignment of targets (B,S) int32 through logp (B,T,V) fp32 on libnbasr, with output frames
+    min(T, output_len_src // len_div) and min(S, targets_len) tokens per row (int64 lengths; all inputs contiguous on one
+    device) -> Alignment.  No host synchronisation."""
+    lib = _lib.load()
+    B, T, V = logp.shape
+    S = targets.shape[1]
+    dev = logp.device
+    with torch.cuda.device(dev):
+        i32 = dict(dtype=torch.int32, device=dev)
+        out = Alignment(torch.empty((B, T), **i32), torch.empty((B, T), **i32), torch.empty((B, S), **i32),
+                        torch.empty((B, S), **i32), torch.empty(B, dtype=torch.float32, device=dev))
+        nwork = lib.nbasr_ctc_align_work_bytes(B, T, S)
+        work = torch.empty(nwork, dtype=torch.uint8, device=dev) if nwork > 0 else None
+        st = torch.cuda.current_stream().cuda_stream
+        _lib.check(lib.nbasr_ctc_align(logp.data_ptr(), B, T, V, targets.data_ptr(), S, output_len_src.data_ptr(), len_div,
+                                       targets_len.data_ptr(), *(t.data_ptr() for t in out),
+                                       work.data_ptr() if work is not None else None, st), 'ctc_align')
+    return out
+
+
 class _CtcLossFn(torch.autograd.Function):
     """Differentiable wrapper for users who call loss() on a tensor that requires grad."""
 
@@ -439,6 +468,25 @@ class Trainer:
                                             ws.dist.data_ptr(), ws.per.data_ptr(), ws.iwork.data_ptr(), st), 'greedy_per')
         self.last_hyp = (ws.hyp, ws.hyp_len, ws.dist)
         return ws.per[0].clone()
+
+    def align(self, output, output_len, val_inputs):
+        """CTC forced alignment of the batch's targets through the log-probs ``output`` (B,T',49) of ``step``; ``output_len``
+        in output frames (one output frame = 4 input frames of 10 ms).  Same arguments as ``decode``:
+            loss, logp, out_len = trainer.step(batch, training=False); ali = trainer.align(logp, out_len, batch)
+        -> trainer.Alignment of device tensors (see ctc_align_cuda).  Target ids outside [1, V) raise ValueError when the
+        targets are host tensors (checked before the upload); on the device such a row comes back with score NaN."""
+        _, (targets, targets_len) = val_inputs
+        V = output.shape[2]
+        if not targets.is_cuda:
+            live = torch.arange(targets.shape[1])[None, :] < torch.as_tensor(targets_len).cpu()[:, None]
+            if bool((((targets < 1) | (targets >= V)) & live).any()):
+                raise ValueError(f'align: target ids must lie in [1, {V})')
+        dev = self.device
+        with torch.cuda.device(dev):
+            return ctc_align_cuda(output.to(device=dev).contiguous().float(),
+                                  output_len.to(device=dev, dtype=torch.int64).contiguous(), 1,
+                                  targets.to(device=dev, dtype=torch.int32).contiguous(),
+                                  targets_len.to(device=dev, dtype=torch.int64).contiguous())
 
     # ---------------------------------------------------------------- epoch loop (trainer.py:80-206)
     def train(self, model, epochs=40, lr=0.0001, reset=False, model_name=None):
