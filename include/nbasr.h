@@ -289,6 +289,31 @@ int nbasr_beam_per(const float* logp, int B, int T, int V, const int64_t* audio_
                    int32_t* raw, int32_t* raw_len, int32_t* hyp, int32_t* hyp_len, int32_t* dist, double* per,
                    int32_t* work, void* stream);
 
+/* Phone error breakdown: the Levenshtein alignment behind nbasr_greedy_per / nbasr_beam_per's dist, per utterance b.
+ *   hyp = hyp[b, :min(H, hyp_len[b])] exactly as those calls write it (folded, no zeros; NOT folded again: the effective
+ *   fold table is not idempotent); ref = targets[b, :min(S, targets_len[b])] mapped through lut (V entries, or NULL) with
+ *   the tokens that map to 0 dropped -- what greedy_per compares against.  n = |hyp|, m = |ref|.
+ *   D(i, j) over hyp prefix i and ref prefix j: D(i, 0) = i, D(0, j) = j,
+ *   D(i, j) = min(D(i-1, j-1) + [hyp[i-1] != ref[j-1]], D(i, j-1) + 1, D(i-1, j) + 1);  D(n, m) = dist.
+ *   A diagonal step is a hit (equal labels) or a substitution, a step j-1 a DELETION (ref token aligned to nothing), a step
+ *   i-1 an INSERTION (hyp token aligned to nothing).  Tie rule: backtrace from (n, m) taking at each cell the first move on
+ *   an optimal path in the order diagonal, deletion, insertion (on the borders the only move) -- among all minimum-cost
+ *   alignments, the one whose move sequence read from the end is lexicographically smallest.
+ * Outputs: counts (B, 4) = [hits, substitutions, deletions, insertions] (hits + S + D = m, hits + S + I = n,
+ * S + D + I = dist); ref_at (B, H) ref position aligned to each hyp position (-1: insertion, and past n); hyp_at (B, S) hyp
+ * position aligned to each ref position (-1: deletion, and past m); positions are those of the compared sequences.
+ * confusion (V, V) is ADDED INTO (sum a corpus over calls): confusion[ref class * V + hyp class] += 1 per aligned pair, row
+ * 0 counting insertions and column 0 deletions.  Integer atomics: deterministic.
+ * A row with a target id outside [0, V) (before or after lut) or a hyp id outside [1, V) is refused on the device: counts
+ * and alignments -1, nothing added to confusion (the call returns 0).  Errors (non-zero return): H or S >= 32 768, V > 64,
+ * or the sequences and three anti-diagonals, H + 7S + 6 bytes, exceeding 220 KB of shared memory.
+ * work: nbasr_edit_align_work_bytes(B, H, S) bytes = 8 * B * (H + S + 1) * ceil((S + 1) / 32) when the backpointers (2 bits
+ * per cell) do not fit in shared memory beside the sequences; 0 otherwise, and work may then be NULL. */
+int nbasr_edit_align(const int32_t* hyp, const int32_t* hyp_len, int H, const int32_t* targets, int S,
+                     const int64_t* targets_len, const int32_t* lut, int B, int V, int32_t* counts, int32_t* ref_at,
+                     int32_t* hyp_at, uint64_t* confusion, void* work, void* stream);
+int64_t nbasr_edit_align_work_bytes(int B, int H, int S);
+
 /* Optimiser tail of Trainer.step (trainer.py:221-225): regulariser 0.01*sum_i ||W_i||_F over the
  * PadConvRelu weights (segments), clip_grad_norm_(5), Adam(eps=1e-7).  Flat fp32 buffers of n
  * elements.  seg_off/seg_len (nseg, int64, device) delimit the regularised tensors.

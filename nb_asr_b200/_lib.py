@@ -81,6 +81,8 @@ _SIGS = {
                          _vp, _vp],
     'nbasr_beam_per': [_vp, C.c_int, C.c_int, C.c_int, _vp, C.c_int, C.c_int, C.c_int, _vp, C.c_int, _vp, _vp, _vp, _vp, _vp, _vp,
                        _vp, _vp, _vp, _vp],
+    'nbasr_edit_align': [_vp, _vp, C.c_int, _vp, C.c_int, _vp, _vp, C.c_int, C.c_int, _vp, _vp, _vp, _vp, _vp, _vp],
+    'nbasr_edit_align_work_bytes': [C.c_int] * 3,
     'nbasr_optim_step': [_vp, _vp, _vp, _vp, _i64, _vp, _vp, C.c_int, _i64, _f32, _f32, _f32, _f32, _f32, _vp, _vp],
     'nbasr_logmel': [_vp, _vp, C.c_int, _i64, _vp, _vp, _vp, _vp, _f32, _vp, C.c_int, _vp, _i64, _vp],
     'nbasr_logmel_work_floats': [C.c_int, _i64],
@@ -124,6 +126,7 @@ def load():
     lib.nbasr_logmel_work_floats.restype = C.c_int64
     lib.nbasr_gate_gram_work_elems.restype = C.c_int64
     lib.nbasr_ctc_align_work_bytes.restype = C.c_int64
+    lib.nbasr_edit_align_work_bytes.restype = C.c_int64
     lib.nbasr_last_error.restype = C.c_char_p
     lib.nbasr_last_error.argtypes = []
     _lib = lib

@@ -21,12 +21,17 @@ import pickle
 from . import PhonemeEncoder, data, distributed, get_loss, get_model, get_trainer, graph_utils, search_space, set_seed
 
 
+ERROR_COLUMNS = ('sub_rate', 'del_rate', 'ins_rate')
+
+
 def evaluate_arch(arch, batches, gpu, precision='bf16', seed=1235, init='reference', conv_gain=1.0, n_ref=None, proxies=(),
-                  proxy_batches=1):
+                  proxy_batches=1, errors=False):
     """One candidate: build from `seed`, eval step (forward + CTC loss) and greedy decode + PER on every batch.
     Returns the reference's epoch metrics (AvgMeter, trainer.py:16-33: unweighted mean of the per-batch means) plus the
     corpus-level PER (sum of edit distances / sum of reference lengths), and for every measure in `proxies` its
-    zero-cost proxy score (nb_asr_b200.proxies) averaged over the first `proxy_batches` batches."""
+    zero-cost proxy score (nb_asr_b200.proxies) averaged over the first `proxy_batches` batches.  `errors`: the decode
+    runs through Trainer.error_report and the row gains the corpus substitution, deletion and insertion rates
+    (ERROR_COLUMNS: summed counts / the sum of reference lengths, the denominator of per_corpus; they add up to it)."""
     if init == 'reference':
         set_seed(seed)
     model = get_model(arch, use_rnn=True, dropout_rate=0.0, gpu=gpu, precision=precision, init=init, seed=seed, conv_gain=conv_gain)
@@ -34,14 +39,22 @@ def evaluate_arch(arch, batches, gpu, precision='bf16', seed=1235, init='referen
     model.engine.max_plans = 64                    # one inference plan per padded length of the evaluation set
     tr = get_trainer((PhonemeEncoder(48), None, None, None), get_loss(), gpus=[gpu], verbose=False)
     tr.model = tr._model = model
-    losses, pers, dists = [], [], []
+    losses, pers, dists, errs = [], [], [], []
     for batch in batches:
         loss, logp, out_len = tr.step(batch, training=False)
-        per = tr.decode(logp, out_len, batch)
+        if errors:
+            rep = tr.error_report(logp, out_len, batch)
+            per = rep.per
+            errs.append(rep.counts[:, 1:].sum(0))
+        else:
+            per = tr.decode(logp, out_len, batch)
         losses.append(loss.double())
         pers.append(per.double())
         dists.append(tr.last_hyp[2].sum().double())
-    res = torch.stack([torch.stack(losses).mean(), torch.stack(pers).mean(), torch.stack(dists).sum()]).tolist()
+    stats = [torch.stack(losses).mean(), torch.stack(pers).mean(), torch.stack(dists).sum()]
+    if errors:
+        stats += list(torch.stack(errs).sum(0).double())
+    res = torch.stack(stats).tolist()
     scores = {}
     if proxies:
         from .proxies import compute_proxies
@@ -53,6 +66,9 @@ def evaluate_arch(arch, batches, gpu, precision='bf16', seed=1235, init='referen
     if n_ref:
         row['per_corpus'] = res[2] / n_ref
     row.update(scores)
+    if errors:
+        n = n_ref or sum(int(tl.sum()) for _, (t, tl) in batches)
+        row.update({c: v / n for c, v in zip(ERROR_COLUMNS, res[3:])})
     return row
 
 
@@ -93,6 +109,9 @@ def build_parser():
                     help='comma-separated zero-cost proxies to add as columns: grad_norm,snip,synflow,jacob_cov,nwot')
     ap.add_argument('--proxy-batches', type=int, default=1,
                     help='the proxies are averaged over the first N batches of the evaluation set')
+    ap.add_argument('--errors', action='store_true',
+                    help='add the corpus substitution, deletion and insertion rates (sub_rate, del_rate, ins_rate: '
+                         'summed counts / summed reference lengths, which add up to per_corpus) as columns')
     return ap
 
 
@@ -134,7 +153,7 @@ def main():
     rows = []
     for i in mine:
         r = evaluate_arch(archs[i], batches, local, args.precision, seed=args.seed, init=args.init, conv_gain=args.conv_gain, n_ref=n_ref,
-                          proxies=args.proxies, proxy_batches=args.proxy_batches)
+                          proxies=args.proxies, proxy_batches=args.proxy_batches, errors=args.errors)
         r['index'] = i
         r['hash'] = graph_utils.get_model_hash(archs[i])
         rows.append(r)
@@ -159,15 +178,16 @@ def main():
         if args.out:
             json.dump(dict(summary=summary, rows=rows), open(args.out, 'w'))
         if args.out_pickle:
+            extra = list(args.proxies) + (list(ERROR_COLUMNS) if args.errors else [])
             header = dict(dataset_type='b200-sweep-eval', version=2, search_space=search_space.get_search_space(),
-                          ops=search_space.all_ops, columns=['model_hash', 'arch_vec', 'ctc_loss', 'per', 'per_corpus'] + list(args.proxies),
+                          ops=search_space.all_ops, columns=['model_hash', 'arch_vec', 'ctc_loss', 'per', 'per_corpus'] + extra,
                           seed=args.seed, precision=args.precision, dataset=args.dataset, utterances=n_utt, init=args.init,
                           conv_gain=summary['conv_gain'], data='synthetic', decode='greedy')
             if args.proxies:
                 header['proxy_batches'] = min(args.proxy_batches, len(batches))
             with open(args.out_pickle, 'wb') as f:
                 pickle.dump(header, f)
-                pickle.dump([[r['hash'], r['arch'], r['loss'], r['per'], r.get('per_corpus')] + [r[m] for m in args.proxies]
+                pickle.dump([[r['hash'], r['arch'], r['loss'], r['per'], r.get('per_corpus')] + [r[m] for m in extra]
                              for r in rows], f)
     if world > 1:
         torch.distributed.destroy_process_group()

@@ -130,6 +130,43 @@ def ctc_align_cuda(logp, output_len_src, len_div, targets, targets_len):
     return out
 
 
+EditAlignment = collections.namedtuple('EditAlignment', 'counts ref_at hyp_at confusion')
+EditAlignment.__doc__ = """Phone error breakdown of a decoded batch (nbasr_edit_align, include/nbasr.h), device tensors:
+counts (B,4) int32 [hits, substitutions, deletions, insertions], ref_at (B,H) int32 reference position aligned to each
+hypothesis position (-1: insertion), hyp_at (B,S) int32 hypothesis position aligned to each reference position (-1:
+deletion), confusion (V,V) int64 view of the uint64 counts confusion[ref class, hyp class] (row 0: insertions, column 0:
+deletions).  A row with an id out of range has counts and alignments -1 and adds nothing to confusion."""
+
+ErrorReport = collections.namedtuple('ErrorReport', 'per counts ref_at hyp_at confusion')
+ErrorReport.__doc__ = """Trainer.error_report: per (the value Trainer.decode returns) and the EditAlignment fields."""
+
+
+def edit_align_cuda(hyp, hyp_len, targets, targets_len, lut, V, confusion=None):
+    """Levenshtein alignment of the folded hypotheses hyp (B,H) int32 / hyp_len (B,) int32, as nbasr_greedy_per writes
+    them, against targets (B,S) int32 / targets_len (B,) int64 mapped through lut (V,) int32 or None, on libnbasr (all
+    inputs contiguous on one device) -> EditAlignment.  confusion: an int64 (V,V) accumulator the counts are added to;
+    None starts from zeros.  No host synchronisation."""
+    lib = _lib.load()
+    B, H = hyp.shape
+    S = targets.shape[1]
+    dev = hyp.device
+    with torch.cuda.device(dev):
+        if confusion is None:
+            confusion = torch.zeros((V, V), dtype=torch.int64, device=dev)
+        elif confusion.shape != (V, V) or confusion.dtype != torch.int64 or confusion.device != dev or not confusion.is_contiguous():
+            raise ValueError(f'edit_align: confusion must be a contiguous int64 ({V}, {V}) tensor on {dev}')
+        i32 = dict(dtype=torch.int32, device=dev)
+        counts, ref_at, hyp_at = torch.empty((B, 4), **i32), torch.empty((B, H), **i32), torch.empty((B, S), **i32)
+        nwork = lib.nbasr_edit_align_work_bytes(B, H, S)
+        work = torch.empty(nwork, dtype=torch.uint8, device=dev) if nwork > 0 else None
+        st = torch.cuda.current_stream().cuda_stream
+        _lib.check(lib.nbasr_edit_align(hyp.data_ptr(), hyp_len.data_ptr(), H, targets.data_ptr(), S, targets_len.data_ptr(),
+                                        lut.data_ptr() if lut is not None else None, B, V, counts.data_ptr(),
+                                        ref_at.data_ptr(), hyp_at.data_ptr(), confusion.data_ptr(),
+                                        work.data_ptr() if work is not None else None, st), 'edit_align')
+    return EditAlignment(counts, ref_at, hyp_at, confusion)
+
+
 class _CtcLossFn(torch.autograd.Function):
     """Differentiable wrapper for users who call loss() on a tensor that requires grad."""
 
@@ -487,6 +524,28 @@ class Trainer:
                                   output_len.to(device=dev, dtype=torch.int64).contiguous(), 1,
                                   targets.to(device=dev, dtype=torch.int32).contiguous(),
                                   targets_len.to(device=dev, dtype=torch.int64).contiguous())
+
+    def error_report(self, output, output_len, val_inputs, beam_width=None):
+        """PER with its breakdown: the decode of ``decode`` (same arguments; ``per`` and ``last_hyp`` are bit-identical to
+        what it gives), then the Levenshtein alignment of every folded hypothesis against its folded reference:
+            loss, logp, out_len = trainer.step(batch, training=False); rep = trainer.error_report(logp, out_len, batch)
+        -> trainer.ErrorReport(per, counts, ref_at, hyp_at, confusion) of device tensors (see edit_align_cuda); the
+        corpus substitution rate is rep.counts[:, 1].sum() / targets_len.sum().  Target ids outside [0, V) raise
+        ValueError when the targets are host tensors (checked before the upload); on the device such a row comes back
+        with counts -1."""
+        _, (targets, targets_len) = val_inputs
+        V = output.shape[2]
+        if not targets.is_cuda:
+            live = torch.arange(targets.shape[1])[None, :] < torch.as_tensor(targets_len).cpu()[:, None]
+            if bool((((targets < 0) | (targets >= V)) & live).any()):
+                raise ValueError(f'error_report: target ids must lie in [0, {V})')
+        dev = self.device
+        with torch.cuda.device(dev):
+            per = self._decode(output, output_len, val_inputs, beam_width)
+            hyp, hyp_len, _ = self.last_hyp
+            ea = edit_align_cuda(hyp, hyp_len, targets.to(device=dev, dtype=torch.int32).contiguous(),
+                                 targets_len.to(device=dev, dtype=torch.int64).contiguous(), self._lut, V)
+        return ErrorReport(per, *ea)
 
     # ---------------------------------------------------------------- epoch loop (trainer.py:80-206)
     def train(self, model, epochs=40, lr=0.0001, reset=False, model_name=None):
