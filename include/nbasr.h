@@ -143,18 +143,6 @@ typedef struct nbasr_gconv {
 } nbasr_gconv;
 
 int nbasr_gconv_fwd(const nbasr_gconv* p, void* stream);
-/* n (1..3) chained grouped-conv edges of one search cell (model.py:49-59: SearchCell.forward runs node 0, 1, 2 in sequence and
- * Node.forward, model.py:13-22, feeds node i+1's op with node i's output): nodes[i+1].x must be nodes[i].epi.out or .out2, all
- * nodes share dtype / B / T / Tp / C / cpg, and every tensor written by the chain is a distinct buffer.  Skip-sum operands
- * (epi.add) may be outputs of earlier nodes of the chain.  Used for the forward node chain and for the input-gradient chain
- * dZ_n -> dZ_{n-1} of the backward pass.
- *   fused = 0: one launch per node, exactly nbasr_gconv_fwd (the default of the engine: measured faster, DESIGN.md 3.2);
- *   fused = 1: ONE persistent launch for the whole chain (tile dependencies between CTAs through flag words in `work`).
- * `work` is a device buffer of nbasr_gconv_chain_work_bytes(...) bytes, zero-filled ONCE by the caller and then owned by the
- * library (it may be shared by every chain launched on one stream); work[2] (uint32) is set if a tile dependency timed out.
- * fp32 / unpacked weights run node by node on the SIMT kernel. */
-int nbasr_gconv_chain(const nbasr_gconv* nodes, int n, int fused, void* work, int64_t work_bytes, void* stream);
-int64_t nbasr_gconv_chain_work_bytes(int B, int T, int C, int cpg, int n);
 int nbasr_pack_gconv_dgrad(const float* w, float* wt, int C, int cpg, int ktaps, void* stream);
 /* bf16 block-diagonal operand for the tcgen05 grouped-conv kernel: [slab][tap][48][64], slabs of 48 (cpg 6/8/12)
  * or 40 (cpg 10) channels; transposed = 1 gives the input-gradient operand (group-transposed, taps flipped).

@@ -7,7 +7,7 @@ from concurrent.futures import ThreadPoolExecutor
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, 'csrc')
 LIB = os.path.join(CSRC, 'libnbasr.so')
-SOURCES = ['api.cu', 'tma_maps.cu', 'gemm_simt.cu', 'gemm2_sm100.cu', 'elementwise.cu', 'layernorm2.cu', 'gconv.cu', 'gconv_sm100.cu', 'gconv_chain_sm100.cu', 'lstm.cu', 'lstm_sm100.cu', 'sequence.cu', 'ctc_align.cu', 'edit_align.cu', 'optim.cu', 'gate_gram.cu', 'pack_batch.cu', 'frontend.cu']
+SOURCES = ['api.cu', 'tma_maps.cu', 'gemm_simt.cu', 'gemm2_sm100.cu', 'elementwise.cu', 'layernorm2.cu', 'gconv.cu', 'gconv_sm100.cu', 'lstm.cu', 'lstm_sm100.cu', 'sequence.cu', 'ctc_align.cu', 'edit_align.cu', 'optim.cu', 'gate_gram.cu', 'pack_batch.cu', 'frontend.cu']
 NVCC_FLAGS = ['-O3', '-std=c++17', '-gencode', 'arch=compute_100a,code=sm_100a', '-lineinfo',
               '-Xcompiler', '-fPIC', '--expt-relaxed-constexpr', '-Xptxas', '-v']
 

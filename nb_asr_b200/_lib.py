@@ -48,8 +48,6 @@ _SIGS = {
     'nbasr_gemm_tn': [C.POINTER(Gemm), _vp],
     'nbasr_gemm_wgrad': [C.POINTER(Wgrad), _vp],
     'nbasr_gconv_fwd': [C.POINTER(GConv), _vp],
-    'nbasr_gconv_chain': [C.POINTER(GConv), C.c_int, C.c_int, _vp, _i64, _vp],
-    'nbasr_gconv_chain_work_bytes': [C.c_int] * 5,
     'nbasr_pack_gconv_dgrad': [_vp, _vp, C.c_int, C.c_int, C.c_int, _vp],
     'nbasr_pack_gconv_mma': [_vp, _vp, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _vp],
     'nbasr_gconv_mma_pack_elems': [C.c_int, C.c_int, C.c_int],
@@ -122,7 +120,6 @@ def load():
         fn.argtypes = args
         fn.restype = C.c_int
     lib.nbasr_gconv_mma_pack_elems.restype = C.c_int64
-    lib.nbasr_gconv_chain_work_bytes.restype = C.c_int64
     lib.nbasr_logmel_work_floats.restype = C.c_int64
     lib.nbasr_gate_gram_work_elems.restype = C.c_int64
     lib.nbasr_ctc_align_work_bytes.restype = C.c_int64

@@ -19,11 +19,10 @@ int nbasr_fail(const char* fmt, ...) {
 namespace {
 struct EnvState {
   bool flag[NBASR_ENV_COUNT];
-  int gemm_bn, gemm_l2pf, chain_dbg;
-  double wgrad_epi_us;
+  int gemm_bn, gemm_l2pf;
   EnvState() {
     static const char* names[NBASR_ENV_COUNT] = {"NBASR_FORCE_SIMT", "NBASR_NO_PDL", "NBASR_GCONV_NO_PREFETCH", "NBASR_LSTM_SS",
-                                                 "NBASR_DEBUG", "NBASR_GEMM_DIRECT_EPI", "NBASR_WGRAD_V1"};
+                                                 "NBASR_DEBUG", "NBASR_GEMM_DIRECT_EPI"};
     for (int i = 0; i < NBASR_ENV_COUNT; ++i) {
       const char* v = getenv(names[i]);      // set and non-empty and not "0"
       flag[i] = v != nullptr && v[0] != 0 && !(v[0] == '0' && v[1] == 0);
@@ -32,10 +31,6 @@ struct EnvState {
     gemm_bn = bn ? atoi(bn) : 0;
     const char* pf = getenv("NBASR_GEMM_L2PF");
     gemm_l2pf = pf ? atoi(pf) : 0;
-    const char* cd = getenv("NBASR_CHAIN_DBG");
-    chain_dbg = cd ? atoi(cd) : 0;
-    const char* eu = getenv("NBASR_WGRAD_EPI_US");
-    wgrad_epi_us = eu ? atof(eu) : 3.0;
   }
 };
 const EnvState g_env;
@@ -43,13 +38,11 @@ const EnvState g_env;
 bool nbasr_env_flag(int which) { return g_env.flag[which]; }
 int nbasr_env_gemm_bn() { return g_env.gemm_bn; }
 int nbasr_env_gemm_l2pf() { return g_env.gemm_l2pf; }
-int nbasr_env_chain_dbg() { return g_env.chain_dbg; }
-double nbasr_env_wgrad_epi_us() { return g_env.wgrad_epi_us; }
 
 extern "C" {
 
 const char* nbasr_last_error(void) { return g_nbasr_err; }
-int nbasr_version(void) { return 100; }
+int nbasr_version(void) { return 101; }
 
 int nbasr_sm_count(void) {
   static int sms = 0;

@@ -247,19 +247,6 @@ int nbasr_gconv_fwd(const nbasr_gconv* p, void* stream) {
   return 0;
 }
 
-int nbasr_gconv_chain(const nbasr_gconv* nodes, int n, int fused, void* work, int64_t work_bytes, void* stream) {
-  NBASR_REQUIRE(nodes != nullptr && n >= 1 && n <= 3, "chain of 1..3 grouped-conv edges");
-  if (nodes[0].B <= 0 || nodes[0].T <= 0) return 0;
-  bool packed = true;
-  for (int i = 0; i < n; ++i) packed = packed && (nodes[i].w_packed & 1) && nodes[i].dtype != NBASR_F32;
-  if (packed) return sm100_gconv_chain(nodes, n, fused, work, work_bytes, as_stream(stream));
-  for (int i = 0; i < n; ++i)       // fp32 / unpacked weights: the SIMT kernel, node by node
-    if (nbasr_gconv_fwd(nodes + i, stream)) return 1;
-  return 0;
-}
-
-int64_t nbasr_gconv_chain_work_bytes(int B, int T, int C, int cpg, int n) { return sm100_gconv_chain_work_bytes(B, T, C, cpg, n); }
-
 int nbasr_pack_gconv_dgrad(const float* w, float* wt, int C, int cpg, int ktaps, void* stream) {
   int total = C * cpg * ktaps;
   pack_gconv_dgrad_kernel<<<(total + 255) / 256, 256, 0, as_stream(stream)>>>(w, wt, C, cpg, ktaps);

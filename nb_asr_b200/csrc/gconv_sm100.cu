@@ -28,11 +28,35 @@
 #include "common.cuh"
 #include "kernels.h"
 #include "sm100_ptx.cuh"
-#include "gconv_sm100.cuh"
 
 using namespace sm100;
 
 namespace {
+
+constexpr int GT = 128;                    // frames per tile
+constexpr int AROWS = 144;                 // 128 + max halo 12, multiple of 8
+constexpr int A_BYTES = AROWS * 128;       // 18432
+constexpr int NW = 48;                     // MMA N (and K window) of a slab
+constexpr int WTAP_BYTES = NW * 128;       // 6144
+constexpr int NSTAGE = 3;                  // (weight-gradient kernel)
+constexpr int NACC = 4;
+constexpr int GC_THREADS = 192;            // weight-gradient kernel: 4 drain warps, producer, MMA
+constexpr int FWD_THREADS = 448;           // forward kernel: 12 epilogue warps, producer, MMA
+constexpr int NEPI = 384;                  // (three column thirds x four TMEM lane quadrants)
+constexpr int OSTAGE_BYTES = GT * NW * 2;  // 12288: bf16 output tile staged for the TMA store
+constexpr int FWD_SMEM_BUDGET = 112 * 1024;
+constexpr int GCONV_SLOTS = 2;             // resident CTAs per SM the grouped-conv kernels size their persistent grids for
+
+__host__ __device__ inline int slab_out(int cpg) { return cpg == 10 ? 40 : 48; }
+// weight-gradient slabs: as many whole groups as fit in 56 channels: 54 / 56 / 50 / 48 for cpg 6 / 8 / 10 / 12 -> fewer,
+// fuller 128-byte loads.  TMA boxes must start on a 16-byte (8-channel) boundary, so the box starts at c0 & ~7 and the
+// slab sits at offset c0 & 7 inside the 64-channel window; channel 63 of the window is never part of a slab and carries
+// the ones column of the fused bias gradient.
+__host__ __device__ inline int wg_slab_out(int cpg) { return (56 / cpg) * cpg; }
+__host__ __device__ inline int fwd_nstage(int ktaps) {
+  int n = (FWD_SMEM_BUDGET - 3072 - ktaps * WTAP_BYTES - 2 * OSTAGE_BYTES) / A_BYTES;
+  return n > 4 ? 4 : n;
+}
 
 struct GcFwdArgs {
   int B, T, C, OUT, ktaps, dstep, off0;
@@ -306,7 +330,7 @@ constexpr int WG_SMEM = NSTAGE * WG_STAGE + 1024 + 256;
 
 struct GcWgArgs {
   int B, T, C, cpg, OUT, ktaps, dstep, off0;
-  int nslabs, nchunks, nunits, nlanes, dbg;
+  int nslabs, nchunks, nunits, nlanes;
   int x_f16;      // X is fp16 holding x / x_scale (the forward's scaled activation): converted to bf16 in shared memory
   float x_scale;
   float* dw;
@@ -383,7 +407,7 @@ gconv_mma_wgrad_kernel(const __grid_constant__ CUtensorMap tmDZ, const __grid_co
         if (elect_one()) {
 #pragma unroll
           for (int k = 0; k < GT / 16; ++k)
-            if (!(p.dbg & 2048) || k == 0) umma_bf16(tm, ad0 + (uint64_t)(k * 128), bd0 + (uint64_t)(k * 128), idesc, (!first || k > 0) ? 1u : 0u);
+            umma_bf16(tm, ad0 + (uint64_t)(k * 128), bd0 + (uint64_t)(k * 128), idesc, (!first || k > 0) ? 1u : 0u);
           umma_commit(empty_bar(stage));
         }
         __syncwarp();
@@ -470,14 +494,12 @@ gconv_mma_wgrad_kernel(const __grid_constant__ CUtensorMap tmDZ, const __grid_co
       }
     }
     named_bar_sync(1, 128);
-    if (!(p.dbg & 1024)) {
-      const int tid = threadIdx.x;                    // 0 .. 127: the drain warps
-      const int nvec = (nrun - head) >> 2, tail = head + 4 * nvec;
-      if (tid < head) atomicAdd(g + tid, run[tid]);
-      for (int j = tid; j < nvec; j += 128)
-        atomicAdd(reinterpret_cast<float4*>(g + head) + j, reinterpret_cast<const float4*>(run + head)[j]);
-      if (tail + tid < nrun) atomicAdd(g + tail + tid, run[tail + tid]);
-    }
+    const int tid = threadIdx.x;                      // 0 .. 127: the drain warps
+    const int nvec = (nrun - head) >> 2, tail = head + 4 * nvec;
+    if (tid < head) atomicAdd(g + tid, run[tid]);
+    for (int j = tid; j < nvec; j += 128)
+      atomicAdd(reinterpret_cast<float4*>(g + head) + j, reinterpret_cast<const float4*>(run + head)[j]);
+    if (tail + tid < nrun) atomicAdd(g + tail + tid, run[tail + tid]);
   }
   tcgen05_fence_before();
   __syncthreads();
@@ -572,7 +594,6 @@ int sm100_gconv_wgrad(const void* dz, const void* x, int x_f16, float x_scale, i
   a.nlanes = std::max(1, std::min(a.nunits, slots / a.nslabs));
   a.dw = dw;
   a.dbias = dbias;
-  a.dbg = nbasr_env_chain_dbg();       // timing experiments only (bits 1024: no gradient atomics, 2048: one MMA per unit)
   CUtensorMap tmDZ, tmX;
   uint64_t dd[3] = {(uint64_t)C, (uint64_t)Tp, (uint64_t)B};
   int64_t sd[3] = {1, C, (int64_t)Tp * C};

@@ -424,150 +424,11 @@ gemm_tn_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
 }
 
 // ---------------------------------------------------------------- weight gradient on CTA pairs (MN-major operands)
-// dW[m, n] += sum_{b,r} dY[(b,r), m] X[(b,r), n]: the pair owns 256 output rows (m) x BN columns over a split of the
-// frame (K) range; each CTA loads its 128 columns of dY and HALF of the X tile per 64-frame K block.
-struct WgArgs2 {
-  int nb, nr, M, N, BN;
-  int m_pairs, n_tiles, chunks_per_utt, total_units, units_per_split;
-  float* dw;
-  int64_t ldw;
-  float* dbias;
-};
-constexpr int WG2_ONES_BYTES = 8192;   // 64 K-rows x 128 B of 1.0 (bias gradient = dY^T 1 via one extra N = 32 MMA)
-constexpr int WG2_SMEM_BYTES = STAGES * STAGE_BYTES + WG2_ONES_BYTES + 1024 + 256;
-constexpr int WG2_THREADS = 192;
-
-__global__ void __launch_bounds__(WG2_THREADS, 1)
-gemm_wgrad_pair_kernel(const __grid_constant__ CUtensorMap tmDY, const __grid_constant__ CUtensorMap tmX, const WgArgs2 p) {
-  extern __shared__ uint8_t smem_raw[];
-  const uint32_t smem_base = (smem_u32(smem_raw) + 1023u) & ~1023u;
-  uint8_t* smem_al = smem_raw + (smem_base - smem_u32(smem_raw));
-  const uint32_t ones_sm = smem_base + STAGES * STAGE_BYTES;
-  const uint32_t bar_base = ones_sm + WG2_ONES_BYTES;
-  auto full_bar = [&](int s) { return bar_base + 8u * s; };
-  auto empty_bar = [&](int s) { return bar_base + 8u * (STAGES + s); };
-  const uint32_t tfull_bar = bar_base + 8u * (2 * STAGES);
-  uint32_t* tmem_ptr_smem = reinterpret_cast<uint32_t*>(smem_al + STAGES * STAGE_BYTES + WG2_ONES_BYTES + 8 * (2 * STAGES + 4));
-  const int warp = threadIdx.x >> 5;
-  const int lane = threadIdx.x & 31;
-  const uint32_t rank = cluster_ctarank();
-  const int pair = blockIdx.x >> 1;
-  const int m0 = (pair % p.m_pairs) * 2 * BM + (int)rank * BM, n0 = (pair / p.m_pairs) * p.BN;
-  const int u_begin = blockIdx.y * p.units_per_split;
-  const int u_end = min(p.total_units, u_begin + p.units_per_split);
-  const int half_bn = p.BN >> 1;
-  const int nbox_b = (half_bn + 63) / 64;             // 64-column boxes of X this CTA loads
-  const bool do_bias = p.dbias != nullptr && n0 == 0;
-  if (do_bias) {
-    uint32_t* o = reinterpret_cast<uint32_t*>(smem_al + STAGES * STAGE_BYTES);
-    for (int i = threadIdx.x; i < WG2_ONES_BYTES / 4; i += blockDim.x) o[i] = 0x3F803F80u;   // bf16 (1.0, 1.0)
-    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-  }
-  if (warp == 0 && lane == 0) {
-    prefetch_tmap(&tmDY);
-    prefetch_tmap(&tmX);
-    for (int s = 0; s < STAGES; ++s) {
-      mbar_init(full_bar(s), 2);
-      mbar_init(empty_bar(s), 1);
-    }
-    mbar_init(tfull_bar, 1);
-    fence_barrier_init();
-  }
-  if (warp == 1) tmem_alloc2(smem_u32(tmem_ptr_smem), 512);
-  pdl_launch_dependents();
-  tcgen05_fence_before();
-  __syncthreads();
-  cluster_sync_all();
-  tcgen05_fence_after();
-  const uint32_t tmem_base = *tmem_ptr_smem;
-  pdl_wait();
-
-  if (u_begin < u_end) {
-    if (warp == 0) {
-      if (lane == 0) {
-        int stage = 0;
-        uint32_t phase = 0;
-        for (int u = u_begin; u < u_end; ++u) {
-          const int b = u / p.chunks_per_utt, r0 = (u % p.chunks_per_utt) * BK;
-          mbar_wait(empty_bar(stage), phase ^ 1);
-          const uint32_t sa = smem_base + stage * STAGE_BYTES;
-          const uint32_t sb = sa + A_STAGE_BYTES;
-          const uint32_t fb = mapa(full_bar(stage), 0);
-          mbar_expect_tx_cluster(fb, (2 + nbox_b) * 64 * 64 * 2);
-          tma2_load_3d(sa, &tmDY, fb, m0, r0, b);
-          tma2_load_3d(sa + 8192, &tmDY, fb, m0 + 64, r0, b);
-          for (int h = 0; h < nbox_b; ++h) tma2_load_3d(sb + h * 8192, &tmX, fb, n0 + (int)rank * half_bn + h * 64, r0, b);
-          if (++stage == STAGES) { stage = 0; phase ^= 1; }
-        }
-      }
-    } else if (warp == 1) {
-      if (lane == 0 && rank == 0) {
-        const uint32_t idesc = make_idesc(2 * BM, p.BN, 1, 1);
-        const uint32_t idesc_ones = make_idesc(2 * BM, 32, 1, 1);
-        int stage = 0;
-        uint32_t phase = 0;
-        for (int u = u_begin; u < u_end; ++u) {
-          mbar_wait(full_bar(stage), phase);
-          tcgen05_fence_after();
-          const uint32_t sa = smem_base + stage * STAGE_BYTES;
-          const uint32_t sb = sa + A_STAGE_BYTES;
-#pragma unroll
-          for (int k = 0; k < BK / 16; ++k) {
-            uint64_t ad = make_smem_desc(sa + k * 2048, 8192, 1024);
-            uint64_t bd = make_smem_desc(sb + k * 2048, 8192, 1024);
-            umma2_bf16(tmem_base, ad, bd, idesc, (u > u_begin || k > 0) ? 1u : 0u);
-            if (do_bias)
-              umma2_bf16(tmem_base + 256, ad, make_smem_desc(ones_sm + k * 2048, 8192, 1024), idesc_ones,
-                         (u > u_begin || k > 0) ? 1u : 0u);
-          }
-          umma2_commit(empty_bar(stage));
-          if (u == u_end - 1) umma2_commit(tfull_bar);
-          if (++stage == STAGES) { stage = 0; phase ^= 1; }
-        }
-      }
-    } else {
-      const int q = warp & 3;
-      const int m = m0 + q * 32 + lane;
-      mbar_wait(tfull_bar, 0);
-      tcgen05_fence_after();
-      const int ncol = min(p.N, n0 + p.BN);
-      if (do_bias) {
-        float one[16];
-        tmem_ld16_nowait(tmem_base + ((uint32_t)(q * 32) << 16) + 256, one);
-        tmem_ld_wait();
-        if (m < p.M) atomicAdd(p.dbias + m, one[0]);
-      }
-      for (int c = 0; c < p.BN; c += 32) {
-        if (n0 + c >= ncol) break;
-        float v[32];
-        tmem_ld32(tmem_base + ((uint32_t)(q * 32) << 16) + c, v);
-        if (m < p.M) {
-          float* dst = p.dw + (int64_t)m * p.ldw + n0 + c;
-#pragma unroll
-          for (int g = 0; g < 8; ++g) {
-            if (n0 + c + g * 4 < ncol)
-              asm volatile("red.global.add.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(dst + g * 4), "f"(v[g * 4]), "f"(v[g * 4 + 1]),
-                           "f"(v[g * 4 + 2]), "f"(v[g * 4 + 3])
-                           : "memory");
-          }
-        }
-      }
-    }
-  }
-  tcgen05_fence_before();
-  __syncthreads();
-  cluster_sync_all();
-  if (warp == 1) {
-    tcgen05_fence_after();
-    tmem_dealloc2(tmem_base, 512);
-  }
-}
-
-// ---------------------------------------------------------------- weight gradient, persistent (round 2)
-// The kernel above pays its set-up (barriers, TMEM allocation, cluster sync, pipeline fill) and its ~3 us fp32 `red.global`
-// drain once per (tile, split) CTA pair -- about half of its time on the step's shapes (ncu r2: tensor pipe 43 % busy, 339
-// CTAs per launch).  Here ONE wave of CTA pairs walks a list of work items (tile, split of the frame range) with TWO TMEM
-// accumulator stages: the drain of item i overlaps the MMAs of item i + 1, and the set-up is paid once.
+// dW[m, n] += sum_{b,r} dY[(b,r), m] X[(b,r), n]: frames are the reduction (K) index.  Persistent: ONE wave of CTA pairs walks
+// a list of work items (tile, split of the frame range) with TWO TMEM accumulator stages, so the drain of item i overlaps the
+// MMAs of item i + 1 and the set-up (barriers, TMEM allocation, cluster sync, pipeline fill) is paid once.  A kernel that pays
+// set-up and its ~3 us fp32 `red.global` drain once per (tile, split) CTA pair spends about half of its time there on the
+// step's shapes (ncu r2: tensor pipe 43 % busy, 339 CTAs per launch).
 //   * tile = 256 output rows (m) x 248 columns (n): the leader CTA feeds N columns 0..127 of the 256-wide MMA, of which
 //     0..119 are X columns n0..n0+119 and 120..127 are (for the first column tile, when a bias gradient is wanted) a
 //     block of ONES planted by a helper warp, so accumulator column 120 = sum_t dY[t][m] = the bias gradient; the peer CTA feeds
@@ -888,7 +749,8 @@ int sm100_gemm_tn_pair(const nbasr_gemm* g, cudaStream_t st) {
   return 0;
 }
 
-static int sm100_gemm_wgrad_persist(const nbasr_wgrad* g, cudaStream_t st) {
+int sm100_gemm_wgrad_pair(const nbasr_wgrad* g, cudaStream_t st) {
+  NBASR_REQUIRE(g->N % 4 == 0 && g->ldw % 4 == 0, "wgrad N / ldw must be multiples of 4");
   WgArgs3 a{};
   a.nb = g->nb; a.nr = g->nr; a.M = g->M; a.N = g->N;
   a.m_pairs = (g->M + 2 * BM - 1) / (2 * BM);
@@ -921,54 +783,5 @@ static int sm100_gemm_wgrad_persist(const nbasr_wgrad* g, cudaStream_t st) {
   }
   cudaError_t e = launch_pdl(gemm_wgrad_persist_kernel, dim3(2 * npairs), dim3(WG3_THREADS), (size_t)WG3_SMEM_BYTES, st, 2, tmDY, tmX, a);
   if (e != cudaSuccess) return nbasr_fail("gemm_wgrad_persist launch: %s", cudaGetErrorString(e));
-  return 0;
-}
-
-int sm100_gemm_wgrad_pair(const nbasr_wgrad* g, cudaStream_t st) {
-  NBASR_REQUIRE(g->N % 4 == 0 && g->ldw % 4 == 0, "wgrad N / ldw must be multiples of 4");
-  if (!nbasr_env_flag(NBASR_ENV_WGRAD_V1)) return sm100_gemm_wgrad_persist(g, st);
-  WgArgs2 a{};
-  a.nb = g->nb; a.nr = g->nr; a.M = g->M; a.N = g->N;
-  a.BN = g->N >= 256 ? 256 : ((g->N + 127) / 128) * 128;      // each CTA loads BN/2 columns in whole 64-column boxes
-  a.m_pairs = (g->M + 2 * BM - 1) / (2 * BM);
-  a.n_tiles = (g->N + a.BN - 1) / a.BN;
-  a.chunks_per_utt = (g->nr + BK - 1) / BK;
-  a.total_units = a.chunks_per_utt * g->nb;
-  const int ctas = 2 * a.m_pairs * a.n_tiles;
-  const int sms = nbasr_sm_count();
-  // split-K factor: minimise  waves x (K blocks per split + epilogue), with 74 co-resident pairs per wave; a K block
-  // (4 MMAs of N/2 cycles) costs ~0.27 us at BN = 256, draining a 128 x BN fp32 tile with red.global ~3 us
-  int splits = 1;
-  {
-    const int pairs = ctas / 2, slots = std::max(1, sms / 2);
-    double best = -1.0;
-    for (int sp = 1; sp <= std::min(a.total_units, 64); ++sp) {
-      const int ups = (a.total_units + sp - 1) / sp;
-      const int eff = (a.total_units + ups - 1) / ups;
-      const int waves = (pairs * eff + slots - 1) / slots;
-      const double epi_us = nbasr_env_wgrad_epi_us();
-      const double cost = waves * (ups * 0.27 * a.BN / 256.0 + epi_us);
-      if (best < 0 || cost < best) { best = cost; splits = eff; }
-    }
-  }
-  a.units_per_split = (a.total_units + splits - 1) / splits;
-  splits = (a.total_units + a.units_per_split - 1) / a.units_per_split;
-  a.dw = g->dw; a.ldw = g->ldw; a.dbias = g->dbias;
-  CUtensorMap tmDY, tmX;
-  uint64_t dd[3] = {(uint64_t)g->M, (uint64_t)g->nr, (uint64_t)g->nb};
-  int64_t sd[3] = {1, g->dy_rs, g->dy_bs};
-  uint32_t bx[3] = {64, BK, 1};
-  if (sm100_get_map(g->dy, 3, dd, sd, bx, &tmDY)) return 1;
-  uint64_t dx[3] = {(uint64_t)g->N, (uint64_t)g->nr, (uint64_t)g->nb};
-  int64_t sx[3] = {1, g->x_rs, g->x_bs};
-  if (sm100_get_map(g->x, 3, dx, sx, bx, &tmX)) return 1;
-  static DevOnce attr;
-  if (!attr) {
-    cudaError_t e = cudaFuncSetAttribute(gemm_wgrad_pair_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, WG2_SMEM_BYTES);
-    if (e != cudaSuccess) return nbasr_fail("gemm_wgrad_pair smem attr: %s", cudaGetErrorString(e));
-    attr = true;
-  }
-  cudaError_t e = launch_pdl(gemm_wgrad_pair_kernel, dim3(ctas, splits), dim3(WG2_THREADS), (size_t)WG2_SMEM_BYTES, st, 2, tmDY, tmX, a);
-  if (e != cudaSuccess) return nbasr_fail("gemm_wgrad_pair launch: %s", cudaGetErrorString(e));
   return 0;
 }

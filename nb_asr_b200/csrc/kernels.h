@@ -7,12 +7,10 @@
 
 // Environment switches are read ONCE, when the library is loaded (api.cu), never on the call path.
 enum NbasrEnvFlag { NBASR_ENV_FORCE_SIMT = 0, NBASR_ENV_NO_PDL, NBASR_ENV_GCONV_NO_PREFETCH, NBASR_ENV_LSTM_SS, NBASR_ENV_DEBUG,
-                    NBASR_ENV_GEMM_DIRECT_EPI, NBASR_ENV_WGRAD_V1, NBASR_ENV_COUNT };
+                    NBASR_ENV_GEMM_DIRECT_EPI, NBASR_ENV_COUNT };
 bool nbasr_env_flag(int which);
 int nbasr_env_gemm_bn();          // NBASR_GEMM_BN tuning override (0 = cost model)
 int nbasr_env_gemm_l2pf();        // NBASR_GEMM_L2PF: K blocks the GEMM producer L2-prefetches ahead of its loads
-int nbasr_env_chain_dbg();        // NBASR_CHAIN_DBG: timing experiments on the chain kernel (bits 1|2: no dependency protocol, 4: strided tiles, 16: general epilogue)
-double nbasr_env_wgrad_epi_us();  // NBASR_WGRAD_EPI_US cost-model constant (default 3.0)
 
 // "Do once per device" latch for cudaFuncSetAttribute(MaxDynamicSharedMemorySize): the attribute is per (function, device),
 // so a process that drives several GPUs (Trainer(gpus=[k]) with k != 0) must opt in on each of them.
@@ -77,9 +75,6 @@ int sm100_get_map(const void* base, int rank, const uint64_t* dims, const int64_
 
 // tcgen05 grouped conv (gconv_sm100.cu)
 int sm100_gconv_fwd(const nbasr_gconv* p, cudaStream_t st);
-// several chained grouped-conv edges in one launch (gconv_chain_sm100.cu)
-int sm100_gconv_chain(const nbasr_gconv* nodes, int n, int fused, void* work, int64_t work_bytes, cudaStream_t st);
-int64_t sm100_gconv_chain_work_bytes(int B, int T, int C, int cpg, int n);
 // x_f16: x is fp16 holding x / x_scale, converted to bf16 in shared memory (otherwise bf16, x_scale unused)
 int sm100_gconv_wgrad(const void* dz, const void* x, int x_f16, float x_scale, int B, int T, int Tp, int C, int cpg, int ktaps,
                       int off0, int dstep, float* dw, float* dbias, cudaStream_t st);

@@ -150,9 +150,6 @@ class Engine:
         self._pack_version = None
         self._bound_ptr = None
         self.training_drop = float(model.dropout_rate)
-        # NBASR_GCONV_CHAIN=1: a cell's chained grouped-conv edges run as ONE persistent launch (nbasr_gconv_chain fused = 1)
-        # (2 / 3: only the forward / only the input-gradient chains -- debugging aid)
-        self.fuse_chains = int(os.environ.get('NBASR_GCONV_CHAIN', '0') or 0)
         self.launches = 0
 
     # ------------------------------------------------------------------ parameter binding
@@ -574,24 +571,6 @@ class Engine:
             call(lst, lib.nbasr_gemm_wgrad, C.byref(w))
             pl.keep.append(w)
 
-        # Chains of grouped-conv edges (a cell's consecutive conv nodes forward, their input gradients backward) go through
-        # nbasr_gconv_chain: one launch per node by default, ONE launch per chain with NBASR_GCONV_CHAIN=1 (measured slower,
-        # DESIGN.md 3.2).  The flag / epoch work buffer is shared by every chain of the plan (one stream).
-        t_blk, tt = [], T
-        for s_ in TR_STRIDES:
-            tt = tt if s_ == 1 else (tt + 1) // 2
-            t_blk.append(tt)
-        wbytes = max(int(lib.nbasr_gconv_chain_work_bytes(B, t_blk[i_], FILTERS[i_], FILTERS[i_] // 100, 3)) for i_ in range(4))
-        pl.chain_work = arena.zeros(((wbytes + 3) // 4,), torch.int32)
-
-        def flush_chain(lst, chain):
-            if not chain:
-                return
-            arr = (GConv * len(chain))(*chain)
-            fused = 1 if self.fuse_chains == 1 or self.fuse_chains == (2 if lst is fwd else 3) else 0
-            call(lst, lib.nbasr_gconv_chain, arr, len(chain), fused, pl.chain_work.data_ptr(), pl.chain_work.numel() * 4)
-            del chain[:]
-
         # ---- input
         pl.audio = arena.zeros((B, FEATURES, T), torch.float32)
         g_in = _Geo(B, T, FEATURES)
@@ -642,7 +621,6 @@ class Engine:
             for ci, cellname in enumerate(self.block_cells[i]):
                 outs = [cur]
                 crec = dict(name=cellname, outs=outs, masks=[], nodes=[])
-                chain = []
                 for n, node in enumerate(arch):
                     op, branches = node[0], node[1:]
                     src = outs[-1]
@@ -651,8 +629,6 @@ class Engine:
                     pn = f'{cellname}.nodes.{n}.op'
                     nrec = dict(op=op, branches=list(branches), pn=pn, mask=None, salt=0)
                     adds = [t.data_ptr() for t in skips]
-                    if op not in CONV_EDGES:
-                        flush_chain(fwd, chain)
                     if op == 'zero':
                         epi = self._epi(Cc, adds=adds, out=o.data_ptr(), fwd=True, copy=cptr(o))
                         call(fwd, lib.nbasr_eltwise, adt, None, Cc, B, Ti, Tp, Cc, C.byref(epi))
@@ -683,12 +659,11 @@ class Engine:
                                 gc.w, gc.w_packed = self.P(pn + '.conv.weight'), 0
                             gc.epi = self._epi(Cc, bias=self.P(pn + '.conv.bias'), relu=1, drop_p=drop_p, salt=sl, adds=adds,
                                                out=o.data_ptr(), mask_out=mask, mask_rows=geo.rows, fwd=True, copy=cptr(o))
-                            chain.append(gc)
+                            call(fwd, lib.nbasr_gconv_fwd, C.byref(gc))
                             pl.keep.append(gc)
                             nrec.update(k=k, d=d, lp=lp)
                     crec['nodes'].append(nrec)
                     outs.append(o)
-                flush_chain(fwd, chain)
                 if m.use_norm:
                     co = zact(geo.rows, Cc, f'b{i}.c{ci}.ln')
                     mean = zbuf(geo.rows, 1, torch.float32)
@@ -768,8 +743,8 @@ class Engine:
         pools = []
         for geo in pl.block_geo:
             pools.append([zbuf(geo.rows, geo.C) for _ in range(5)])
-        # one dZ buffer per node: a chain writes dZ_{j-1} while neighbouring CTAs still read dZ_j, and the weight gradients of
-        # the whole chain run after it
+        # one dZ buffer per node: the weight gradients of a cell's consecutive conv nodes run after all of their input
+        # gradients and read every node's dZ
         dzs = [[zbuf(geo.rows, geo.C) for _ in range(max(2, len(arch)))] for geo in pl.block_geo]
 
         gout = pools[3].pop()
@@ -866,11 +841,10 @@ class Engine:
                         epi = self._epi(Cc, out2=dz_t.data_ptr(), mask2=last['mask'], scale2=dscale, mask_rows=geo.rows)
                         call(bwd, lib.nbasr_eltwise, dt, gout.data_ptr(), Cc, B, Ti, Tp, Cc, C.byref(epi))
                         pl.keep.append(epi)
-                chain, chain_wg = [], []
+                chain_wg = []
 
                 def flush_bwd():
-                    # input-gradient chain first (it produces the dZ of every node), then the chain's weight gradients
-                    flush_chain(bwd, chain)
+                    # weight gradients of the conv nodes since the last flush, after all of their input gradients
                     for a_ in chain_wg:
                         call(bwd, lib.nbasr_gconv_wgrad_x, *a_)
                     del chain_wg[:]
@@ -914,7 +888,7 @@ class Engine:
                         gc.ktaps, gc.off0, gc.dstep, gc.w = k, lp - (k - 1) * dd, dd, self.wt[pn].data_ptr()
                         gc.w_packed = 3 if dt == BF16 else 0      # packed | stable
                         gc.epi = epi
-                        chain.append(gc)
+                        call(bwd, lib.nbasr_gconv_fwd, C.byref(gc))
                         pl.keep.append(gc)
                 flush_bwd()
                 for k in range(1, nn_ + 1):   # (without norm, g[nn_] is the consumed incoming buffer)
@@ -974,15 +948,12 @@ class Engine:
     # ------------------------------------------------------------------ execution
     def _run(self, ops):
         st = torch.cuda.current_stream().cuda_stream
-        n = 0
-        chain = self.lib.nbasr_gconv_chain
         for fn, args in ops:
             rc = fn(*args, st)
             if rc != 0:
                 raise _lib.NbasrError(f'{fn.__name__}: {self.lib.nbasr_last_error().decode()}')
-            # kernels launched: every C-ABI call launches >= 1 kernel of libnbasr; an unfused chain launches one per node
-            n += args[1] if (fn is chain and not args[2]) else 1
-        self.launches += n
+        # kernels launched: every C-ABI call launches >= 1 kernel of libnbasr
+        self.launches += len(ops)
 
     @_on_device
     def forward(self, audio, training=None, grad=None, input_grad=False):

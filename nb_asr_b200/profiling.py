@@ -4,7 +4,6 @@ Used by bench.py for the live roofline figure and by tools/ for optimisation wor
 FLOPs / bytes follow SURVEY.md §8(d) / DESIGN.md "Kernels and rooflines".
 """
 import collections
-import ctypes as C
 
 import torch
 
@@ -43,14 +42,6 @@ def op_work(fn_name, args, es):
         n_t = 1 + g.epi.n_add + (1 if g.epi.out else 0) + (1 if (g.epi.out2 and g.epi.mask2) else 0)     # tensors read/written once
         n_m = (1 if g.epi.mask_out else 0) + (1 if g.epi.mask2 else 0)                 # 1 bit / element each
         return f'gconv C={g.C} k={g.ktaps} d={g.dstep}', 2.0 * el * g.cpg * g.ktaps, el * es * n_t + el * n_m / 8.0
-    if fn_name == 'nbasr_gconv_chain':
-        # a chain launch processes n nodes: algorithmic work = the sum of its nodes' (SURVEY.md 8d per-node figures)
-        fl = by = 0.0
-        for i in range(args[1]):
-            _, f1, b1 = op_work('nbasr_gconv_fwd', (C.byref(args[0][i]),), es)
-            fl, by = fl + f1, by + b1
-        g = args[0][0]
-        return f'gconv C={g.C} chain of {args[1]}', fl, by
     if fn_name in ('nbasr_gconv_wgrad', 'nbasr_gconv_wgrad_x'):
         B, T, Tp, Cc, cpg, k = args[3:9] if fn_name == 'nbasr_gconv_wgrad' else args[5:11]
         el = B * T * Cc
@@ -74,8 +65,6 @@ def op_work(fn_name, args, es):
 def gconv_issue_floor_cycles(fn_name, args):
     """Structural floor of the tcgen05 grouped-conv forward / input-gradient kernel (DESIGN.md 3.1): 3*k MMAs of N = 48 per
     128-frame x 48-channel tile, each >= 88 cycles of tensor-pipe issue (both operands in shared memory), on one SM."""
-    if fn_name == 'nbasr_gconv_chain':
-        return sum(gconv_issue_floor_cycles('nbasr_gconv_fwd', (C.byref(args[0][i]),)) for i in range(args[1]))
     if fn_name != 'nbasr_gconv_fwd':
         return 0.0
     g = _struct_of(args[0], GConv)
@@ -103,8 +92,7 @@ def profile_ops(engine, ops, iters=3):
             tag, fl, by = op_work(fn.__name__, args, es)
             d = acc.setdefault(tag, dict(n=0, ms=0.0, flops=0.0, bytes=0.0, floor_cycles=0.0))
             d['floor_cycles'] += gconv_issue_floor_cycles(fn.__name__, args)
-            # kernel launches of this entry (an unfused grouped-conv chain launches one kernel per node)
-            d['n'] += args[1] if (fn.__name__ == 'nbasr_gconv_chain' and not args[2]) else 1
+            d['n'] += 1
             d['ms'] += evs[i].elapsed_time(evs[i + 1])
             d['flops'] += fl
             d['bytes'] += by

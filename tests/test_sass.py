@@ -20,7 +20,6 @@ EXPECT = {
     'gemm_wgrad_persist_kernel': ['UTCHMMA', 'UTMALDG', 'LDTM', 'UTCBAR'],
     'gconv_mma_fwd_kernel': ['UTCHMMA', 'UTMALDG', 'UTMASTG', 'LDTM'],
     'gconv_mma_wgrad_kernel': ['UTCHMMA', 'UTMALDG', 'LDTM'],
-    'gconv_chain_kernel': ['UTCHMMA', 'UTMALDG', 'UTMASTG', 'LDTM'],
     'lstm_cluster_fwd_kernelILb1': ['UTCHMMA', 'UTMALDG', 'STTM', 'LDTM', 'UBLKCP'],   # W slice in tensor memory, DSMEM bulk copies
     'lstm_cluster_bwd_kernel': ['UTCHMMA', 'UTMALDG', 'STTM', 'LDTM', 'UBLKCP'],
 }

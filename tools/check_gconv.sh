@@ -1,12 +1,2 @@
 #!/bin/bash
-timeout 600 python -m pytest tests/test_gpu_1_kernels.py tests/test_gpu_8_gconv_chain.py -m gpu -x -q -k "gconv or chain" 2>&1 | tail -4
-python tools/one_chain.py
-OPS=conv7d2,conv7d2,conv7d2 SKIPS=1 python tools/one_chain.py
-BWD=1 python tools/one_chain.py
-for arch in default c7d2_skips; do
-  timeout 300 python bench.py --arch $arch --steps 10 --warmup 3 --profile --no-cpu-baseline --no-extra 2>gpurun_out/g12_prof_$arch.txt | python -c "
-import json,sys
-d=json.loads(sys.stdin.read().strip().splitlines()[-1])
-f=d['roofline']['families']
-print('$arch', 'step', round(d['ms_per_step'],3), 'e2e', round(d['e2e']['ms_per_step'],3), {k:(v['ms'],v['n']) for k,v in f.items() if 'gconv' in k})"
-done
+timeout 600 python -m pytest tests/test_gpu_1_kernels.py -m gpu -x -q -k gconv 2>&1 | tail -4
