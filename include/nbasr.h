@@ -320,6 +320,15 @@ int nbasr_optim_step(float* param, float* grad, float* m, float* v, int64_t n, c
 int nbasr_param_stats(const float* param, const float* grad, const int64_t* seg_off, const int64_t* seg_len, int nseg,
                       int64_t seg_chunks, double* part, double* out, void* stream);
 
+/* Gradient signal-to-noise of the ZiCo proxy (Li et al. 2023) over N gradient samples of the same flat buffer
+ * (2 <= N <= 16; other N is an error): sample k of parameter i is g[k*g_stride + i].  Per parameter, in fp64:
+ *   m = sum_k g_k / N,  var = sum_k (g_k - m)^2 / N,  included iff var > 0 (the samples are not all equal),
+ *   r = (sum_k |g_k| / N) / sqrt(var).
+ * out[2*s] = sum of r over the included parameters of segment s, out[2*s + 1] = their number (an exact double).
+ * Segment table, part (2 * seg_chunks doubles) and determinism as in nbasr_param_stats. */
+int nbasr_grad_snr(const float* g, int64_t g_stride, int N, const int64_t* seg_off, const int64_t* seg_len, int nseg,
+                   int64_t seg_chunks, double* part, double* out, void* stream);
+
 /* Row Gram matrix and row sums of a (B, D) fp32 matrix with row pitch ld (B <= 128), in fp64:
  * gram[i*B + j] = sum_d x[i*ld + d] * x[j*ld + d],  rowsum[i] = sum_d x[i*ld + d].
  * work: ceil(D / 256) * (B*(B+1)/2 + B) doubles.  Deterministic (256-column chunks summed in chunk order).

@@ -61,6 +61,7 @@ _SIGS = {
     'nbasr_transpose_in': [_vp, _vp, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _f32, _vp],
     'nbasr_transpose_out': [_vp, _vp, C.c_int, C.c_int, C.c_int, C.c_int, _vp],
     'nbasr_param_stats': [_vp, _vp, _vp, _vp, C.c_int, _i64, _vp, _vp, _vp],
+    'nbasr_grad_snr': [_vp, _i64, C.c_int, _vp, _vp, C.c_int, _i64, _vp, _vp, _vp],
     'nbasr_row_gram': [_vp, C.c_int, _i64, _i64, _vp, _vp, _vp, _vp],
     'nbasr_gate_gram': [_vp, C.c_int, _vp, C.c_int, _vp, _vp, _vp],
     'nbasr_gate_gram_work_elems': [C.c_int],

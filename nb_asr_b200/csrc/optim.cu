@@ -129,6 +129,70 @@ __global__ void seg_stats_kernel(const float* __restrict__ p, const float* __res
   }
 }
 
+// Gradient signal-to-noise of the ZiCo proxy (nbasr_grad_snr): parameter i of a segment has the N fp32 samples
+// g[k * g_stride + i]; with m = S / N and var = sum_k (g_k - m)^2 / N (population), r = (A / N) / sqrt(var) when var > 0.
+// In fp64 the kernel forms S = sum_k g_k, A = sum_k |g_k| and Q = sum_k (N g_k - S)^2 = N^3 var, and r = sqrt(N) A / sqrt(Q)
+// (one reciprocal square root per parameter instead of three divisions and a square root).  For one chunk: sum r ->
+// part[blk], number of parameters with Q > 0 -> part[nchunks + blk].  N g_k is exact (24 + 4 significant bits); N equal
+// samples sum exactly to N g, so Q = 0; samples that are not all equal leave some N g_k - S != 0, whose square is far
+// above fp64's underflow.  So Q > 0 exactly when the samples are not all equal -- the same set as var > 0 in a numpy
+// restatement on the same samples.
+constexpr int SNR_MAX_N = 16;
+
+// NMAX >= N samples per parameter, VEC = 16 / NMAX parameters per thread and step (elements i, i + 256, ... of the
+// chunk): the 16 loads of a step are issued together, so a small N still keeps enough bytes in flight.
+template <int NMAX>
+__global__ void __launch_bounds__(256) seg_snr_kernel(const float* __restrict__ g, int64_t g_stride, int N,
+                                                      const int64_t* __restrict__ off, const int64_t* __restrict__ len,
+                                                      int nseg, int64_t nchunks, double* __restrict__ part) {
+  constexpr int VEC = SNR_MAX_N / NMAX;
+  int s; int64_t start;
+  if (!seg_locate(len, nseg, blockIdx.x, s, start)) return;
+  const float* x = g + off[s] + start;
+  const int n = (int)(min(len[s], start + SEG_CHUNK) - start);
+  const double dn = N, sqrt_n = sqrt(dn);
+  double rsum = 0.0, cnt = 0.0;
+  for (int i0 = threadIdx.x; i0 < n; i0 += VEC * blockDim.x) {
+    float v[VEC][NMAX];
+#pragma unroll
+    for (int j = 0; j < VEC; ++j) {
+      const int i = i0 + j * blockDim.x;
+#pragma unroll
+      for (int k = 0; k < NMAX; ++k) v[j][k] = (k < N && i < n) ? x[k * g_stride + i] : 0.f;
+    }
+#pragma unroll
+    for (int j = 0; j < VEC; ++j) {
+      if (i0 + j * (int)blockDim.x >= n) break;
+      double S = 0.0, A = 0.0;
+#pragma unroll
+      for (int k = 0; k < NMAX; ++k) {
+        if (k < N) {
+          S += v[j][k];
+          A += fabs((double)v[j][k]);
+        }
+      }
+      double Q = 0.0;
+#pragma unroll
+      for (int k = 0; k < NMAX; ++k) {
+        if (k < N) {
+          const double d = fma(dn, (double)v[j][k], -S);
+          Q = fma(d, d, Q);
+        }
+      }
+      if (Q > 0.0) {
+        rsum = fma(sqrt_n * A, rsqrt(Q), rsum);
+        cnt += 1.0;
+      }
+    }
+  }
+  rsum = block_sum(rsum);
+  cnt = block_sum(cnt);
+  if (threadIdx.x == 0) {
+    part[blockIdx.x] = rsum;
+    part[nchunks + blockIdx.x] = cnt;
+  }
+}
+
 // Row Gram matrix of nbasr_row_gram: block c covers columns [c * GRAM_CHUNK, (c + 1) * GRAM_CHUNK) of every row and writes
 // the fp64 partials of the upper triangle G[i][j] (i <= j, row-major triangle order) and of the row sums.
 constexpr int GRAM_CHUNK = 256;
@@ -311,6 +375,28 @@ extern "C" int nbasr_param_stats(const float* param, const float* grad, const in
   NBASR_REQUIRE(seg_chunks > 0, "seg_chunks = sum of ceil(seg_len / 16384)");
   cudaStream_t st = as_stream(stream);
   seg_stats_kernel<<<(unsigned)seg_chunks, 256, 0, st>>>(param, grad, seg_off, seg_len, nseg, seg_chunks, part);
+  NBASR_CHECK_LAUNCH();
+  seg_reduce_kernel<double><<<dim3(nseg, 2), 256, 0, st>>>(part, seg_len, nseg, out, seg_chunks, 2);
+  NBASR_CHECK_LAUNCH();
+  return 0;
+}
+
+extern "C" int nbasr_grad_snr(const float* g, int64_t g_stride, int N, const int64_t* seg_off, const int64_t* seg_len,
+                              int nseg, int64_t seg_chunks, double* part, double* out, void* stream) {
+  NBASR_REQUIRE(N >= 2 && N <= SNR_MAX_N, "2 <= N <= 16 gradient samples");
+  if (nseg <= 0) return 0;
+  NBASR_REQUIRE(seg_chunks > 0, "seg_chunks = sum of ceil(seg_len / 16384)");
+  NBASR_REQUIRE(g_stride >= 0, "snapshot stride");
+  cudaStream_t st = as_stream(stream);
+  const unsigned grid = (unsigned)seg_chunks;
+  if (N == 2)
+    seg_snr_kernel<2><<<grid, 256, 0, st>>>(g, g_stride, N, seg_off, seg_len, nseg, seg_chunks, part);
+  else if (N <= 4)
+    seg_snr_kernel<4><<<grid, 256, 0, st>>>(g, g_stride, N, seg_off, seg_len, nseg, seg_chunks, part);
+  else if (N <= 8)
+    seg_snr_kernel<8><<<grid, 256, 0, st>>>(g, g_stride, N, seg_off, seg_len, nseg, seg_chunks, part);
+  else
+    seg_snr_kernel<16><<<grid, 256, 0, st>>>(g, g_stride, N, seg_off, seg_len, nseg, seg_chunks, part);
   NBASR_CHECK_LAUNCH();
   seg_reduce_kernel<double><<<dim3(nseg, 2), 256, 0, st>>>(part, seg_len, nseg, out, seg_chunks, 2);
   NBASR_CHECK_LAUNCH();

@@ -16,7 +16,14 @@ NAS-Bench-ASR users' proxy code computes them through ``get_prunable_copy``).
   score log|det K| (fp64 slogdet on the host; -inf when K is singular, e.g. for a batch with a duplicated utterance).
   Valid frames of block k: min(T_k, ceil(audio_len / 2^s_k)), s = (0, 0, 1, 2).  K comes from the gate-bit masks a
   grad plan's forward pass already writes (nbasr_gate_gram, exact integer counts); with grad_norm / snip it reuses
-  their forward pass.
+  their forward pass;
+* zico (ZiCo, Li et al. 2023; opt-in by name, not in MEASURES): the batch is cut into N interleaved splits (utterance b
+  goes to split b mod N, each keeps the padded T); g_k is the gradient of split k's CTC loss (as grad_norm's, dropout
+  off).  Per parameter, in fp64, m = mean_k g_k, var = mean_k (g_k - m)^2 and, where var > 0 (the N samples are not all
+  equal), r = mean_k |g_k| / sqrt(var); R_l = sum r over tensor l and the score is the sum of ln R_l over the tensors
+  with R_l > 0 (nbasr_grad_snr over the N snapshots of the flat gradient buffer).  The ratio is large exactly where the
+  split gradients nearly agree, so it amplifies the fp32-atomic rounding of the weight-gradient kernels: two runs agree
+  less closely than the other measures do (DESIGN.md 7b).
 
 Scored tensors are the ``.weight`` of every Conv1d and Linear (time-reduction and grouped convs, linear edges, classifier);
 LSTM, LayerNorm and biases are not scored ("conv and linear layers", as in the pruning-at-init library).  Per-tensor sums
@@ -33,8 +40,10 @@ from . import _lib
 from .model import ASRModel, FEATURES, TR_STRIDES
 from .trainer import ctc_loss_cuda
 
-MEASURES = ('grad_norm', 'snip', 'synflow', 'jacob_cov', 'nwot')
-SEG_CHUNK = 16384          # chunk of nbasr_param_stats (optim.cu)
+MEASURES = ('grad_norm', 'snip', 'synflow', 'jacob_cov', 'nwot')     # the default set
+ACCEPTED = MEASURES + ('zico',)                                        # every measure compute_proxies computes by name
+SEG_CHUNK = 16384          # chunk of nbasr_param_stats / nbasr_grad_snr (optim.cu)
+ZICO_MAX_SPLITS = 16       # N <= 16 gradient samples per parameter (nbasr_grad_snr)
 # s_k of block k: its frames are the input's halved s_k times, (0, 0, 1, 2)
 LEN_SHIFT = tuple(sum(1 for s in TR_STRIDES[:k + 1] if s == 2) for k in range(len(TR_STRIDES)))
 
@@ -42,9 +51,9 @@ LEN_SHIFT = tuple(sum(1 for s in TR_STRIDES[:k + 1] if s == 2) for k in range(le
 def parse_measures(text):
     """'grad_norm,snip' -> ('grad_norm', 'snip'); unknown names raise ValueError."""
     names = tuple(n.strip() for n in text.split(',') if n.strip())
-    bad = [n for n in names if n not in MEASURES]
+    bad = [n for n in names if n not in ACCEPTED]
     if bad or not names:
-        raise ValueError(f'unknown proxy measure(s) {bad or text!r}; choose from {",".join(MEASURES)}')
+        raise ValueError(f'unknown proxy measure(s) {bad or text!r}; choose from {",".join(ACCEPTED)}')
     return names
 
 
@@ -53,8 +62,9 @@ def scored_names(model):
     return [f'{n}.weight' for n, m in model.named_modules() if isinstance(m, (nn.Conv1d, nn.Linear))]
 
 
-def _param_stats(eng, names):
-    """{name: (sum g^2, sum |theta g|)} over the engine's flat buffers, fp64."""
+def _segments(eng, names):
+    """Segment table of the named tensors in the engine's flat buffers for nbasr_param_stats / nbasr_grad_snr:
+    (offsets, lengths, chunk count, partials, out (nseg, 2) fp64), all on the device."""
     segs = [eng.slices[n] for n in names]
     dev = eng.device
     off = torch.tensor([o for o, _ in segs], dtype=torch.int64, device=dev)
@@ -62,11 +72,72 @@ def _param_stats(eng, names):
     chunks = sum((n + SEG_CHUNK - 1) // SEG_CHUNK for _, n in segs)
     part = torch.empty(2 * chunks, dtype=torch.float64, device=dev)
     out = torch.empty(len(segs), 2, dtype=torch.float64, device=dev)
+    return off, ln, chunks, part, out
+
+
+def _param_stats(eng, names):
+    """{name: (sum g^2, sum |theta g|)} over the engine's flat buffers, fp64."""
+    off, ln, chunks, part, out = _segments(eng, names)
     st = torch.cuda.current_stream().cuda_stream
-    _lib.check(eng.lib.nbasr_param_stats(eng.flat_p.data_ptr(), eng.flat_g.data_ptr(), off.data_ptr(), ln.data_ptr(), len(segs),
+    _lib.check(eng.lib.nbasr_param_stats(eng.flat_p.data_ptr(), eng.flat_g.data_ptr(), off.data_ptr(), ln.data_ptr(), len(names),
                                          chunks, part.data_ptr(), out.data_ptr(), st), 'param_stats')
     vals = out.cpu().tolist()
     return {n: tuple(v) for n, v in zip(names, vals)}
+
+
+def zico_split(batch, splits):
+    """The N = `splits` interleaved splits of batch ((audio, audio_len), (targets, targets_len)): utterance b goes to split
+    b mod N (the sweep's batches are length-sorted: contiguous slices would differ systematically in length); every split
+    keeps the batch's padded T.  2 <= N <= min(B, 16), else ValueError."""
+    (audio, audio_len), (targets, targets_len) = batch
+    B = audio.shape[0]
+    if not 2 <= splits <= min(B, ZICO_MAX_SPLITS):
+        raise ValueError(f'zico needs 2 <= splits <= min(B, {ZICO_MAX_SPLITS}) = {min(B, ZICO_MAX_SPLITS)}, got {splits}')
+    return [((audio[k::splits], audio_len[k::splits]), (targets[k::splits], targets_len[k::splits])) for k in range(splits)]
+
+
+def zico_snapshots(model, batch, splits=2):
+    """(N, len(flat_g)) fp32 device tensor: row k is the engine's flat gradient of the CTC loss of split k of `batch`
+    (zico_split; one forward + backward of a grad plan per split, dropout off).  The model's flat_g is unchanged."""
+    parts = zico_split(batch, splits)
+    eng = model.engine
+    eng.bind()
+    dev = eng.device
+    with torch.cuda.device(dev):
+        snaps = torch.empty(splits, eng.flat_g.numel(), dtype=torch.float32, device=dev)
+        saved_g = eng.flat_g.clone()
+        try:
+            for k, ((audio, audio_len), (targets, targets_len)) in enumerate(parts):
+                pl = eng.forward(audio.to(dev, torch.float32).contiguous(), training=False, grad=True)
+                ctc_loss_cuda(pl.logp, audio_len.to(dev, torch.int64).contiguous(), 4,
+                              targets.to(dev, torch.int32).contiguous(), targets_len.to(dev, torch.int64).contiguous(),
+                              dlogits=pl.dlogits)
+                eng.backward(pl)
+                snaps[k].copy_(eng.flat_g)
+        finally:
+            eng.flat_g.copy_(saved_g)
+    return snaps
+
+
+def zico_stats(model, snaps):
+    """{scored name: (R, n)} from gradient snapshots (N, len(flat_g)): R = sum of mean|g| / std(g) over the n parameters
+    whose N samples are not all equal (nbasr_grad_snr, fp64, deterministic)."""
+    eng = model.engine
+    names = scored_names(model)
+    if snaps.dtype != torch.float32 or snaps.dim() != 2 or snaps.stride(1) != 1 or snaps.shape[1] < eng.flat_g.numel():
+        raise ValueError('snapshots: a (N, len(flat_g)) fp32 tensor with unit column stride')
+    with torch.cuda.device(eng.device):
+        off, ln, chunks, part, out = _segments(eng, names)
+        _lib.check(eng.lib.nbasr_grad_snr(snaps.data_ptr(), snaps.stride(0), snaps.shape[0], off.data_ptr(), ln.data_ptr(),
+                                          len(names), chunks, part.data_ptr(), out.data_ptr(),
+                                          torch.cuda.current_stream().cuda_stream), 'grad_snr')
+        vals = out.cpu().tolist()
+    return {n: tuple(v) for n, v in zip(names, vals)}
+
+
+def zico_layers(stats):
+    """{name: ln R} over the tensors with R > 0 (a tensor with no included parameter contributes nothing)."""
+    return {n: math.log(r) for n, (r, _) in stats.items() if r > 0}
 
 
 def corrcoef_from_gram(G, s, D):
@@ -195,15 +266,18 @@ def synflow_stats(model, T, copy=None):
     return {n: v[1] for n, v in st.items()}
 
 
-def compute_proxies(model, batch, measures=MEASURES, per_layer=False):
-    """Zero-cost proxies of `model` on one batch ((audio (B,80,T), audio_len), (targets, targets_len)).
+def compute_proxies(model, batch, measures=MEASURES, per_layer=False, zico_splits=2):
+    """Zero-cost proxies of `model` on one batch ((audio (B,80,T), audio_len), (targets, targets_len)).  `measures`: names
+    from ACCEPTED (default MEASURES; zico only when named, over `zico_splits` interleaved splits).
 
-    Returns {measure: float}, or with per_layer=True {measure: {parameter name: float}} for grad_norm / snip / synflow
-    (jacob_cov and nwot are whole-network scores and stay floats)."""
+    Returns {measure: float}, or with per_layer=True {measure: {parameter name: float}} for grad_norm / snip / synflow /
+    zico (zico: ln R of the contributing tensors only; jacob_cov and nwot are whole-network scores and stay floats)."""
     measures = tuple(measures)
-    bad = [m for m in measures if m not in MEASURES]
+    bad = [m for m in measures if m not in ACCEPTED]
     if bad:
-        raise ValueError(f'unknown proxy measure(s) {bad}; choose from {MEASURES}')
+        raise ValueError(f'unknown proxy measure(s) {bad}; choose from {ACCEPTED}')
+    if 'zico' in measures:
+        zico_split(batch, zico_splits)               # an invalid split count fails before any GPU work
     eng = model.engine
     eng.bind()
     dev = eng.device
@@ -237,6 +311,9 @@ def compute_proxies(model, batch, measures=MEASURES, per_layer=False):
             eng.flat_g.copy_(saved_g)
         if 'synflow' in measures:
             out['synflow'] = synflow_stats(model, audio.shape[2])
+        if 'zico' in measures:
+            # after the other measures: their plans and passes run exactly as without zico
+            out['zico'] = zico_layers(zico_stats(model, zico_snapshots(model, batch, zico_splits)))
     res = {}
     for m in measures:
         v = out[m]

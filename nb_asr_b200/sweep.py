@@ -73,7 +73,7 @@ def evaluate_arch(arch, batches, gpu, precision='bf16', seed=1235, init='referen
 
 
 def proxy_list(text):
-    """argparse type of --proxies: comma-separated measure names of nb_asr_b200.proxies.MEASURES."""
+    """argparse type of --proxies: comma-separated measure names of nb_asr_b200.proxies.ACCEPTED."""
     from .proxies import parse_measures
     try:
         return parse_measures(text)
@@ -106,7 +106,8 @@ def build_parser():
     ap.add_argument('--out-pickle', default=None, help='nb-asr style table: header, then rows')
     ap.add_argument('--all', action='store_true', help='evaluate every arch_vec, not one per isomorphism class')
     ap.add_argument('--proxies', type=proxy_list, default=(),
-                    help='comma-separated zero-cost proxies to add as columns: grad_norm,snip,synflow,jacob_cov,nwot')
+                    help='comma-separated zero-cost proxies to add as columns: grad_norm,snip,synflow,jacob_cov,nwot,zico '
+                         '(zico: gradient signal-to-noise over two interleaved halves of each batch)')
     ap.add_argument('--proxy-batches', type=int, default=1,
                     help='the proxies are averaged over the first N batches of the evaluation set')
     ap.add_argument('--errors', action='store_true',

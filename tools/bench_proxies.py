@@ -3,9 +3,12 @@
     python tools/bench_proxies.py [--reps 5] [--sample 24] [--out profiles/proxies.json]
 
 * ms per measure (grad_norm and snip share one forward + backward and are timed together) for four archs at B x T = 64 x 500;
-  nwot alone (one forward pass + nbasr_gate_gram) and grad_norm + snip + nwot (nwot reuses their forward pass);
+  nwot alone (one forward pass + nbasr_gate_gram) and grad_norm + snip + nwot (nwot reuses their forward pass); zico
+  alone (two half-batch forward + backward passes + nbasr_grad_snr);
+* nbasr_grad_snr alone (CUDA events) on each arch's own two gradient snapshots (N = 2) and the bytes it reads;
 * the sweep's candidates per second on a fixed sample of unique archs (every k-th of the 8 242), evaluated exactly as
-  nb_asr_b200.sweep does, without proxies, with --proxies nwot and with all five proxies (--proxy-batches 1);
+  nb_asr_b200.sweep does, without proxies, with --proxies nwot, with all five proxies and with --proxies zico
+  (--proxy-batches 1), and the Kendall tau between the zico columns of the 16-bit and the fp32 sweep;
 * the GPU's name and power limit, read in the same run.
 """
 import argparse
@@ -19,12 +22,12 @@ import torch
 
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import nb_asr_b200 as nb  # noqa: E402
-from nb_asr_b200 import data, graph_utils, proxies, sweep  # noqa: E402
+from nb_asr_b200 import _lib, data, graph_utils, proxies, sweep  # noqa: E402
 
 ARCHS = {'default': [[1, 0], [1, 0, 0], [1, 0, 0, 0]], 'linear_skips': [[0, 1], [0, 1, 1], [0, 1, 1, 1]],
          'c7d2_skips': [[4, 1], [4, 1, 1], [4, 1, 1, 1]], 'zero_mix': [[5, 1], [1, 1, 0], [5, 0, 1, 1]]}
 GROUPS = {'grad_norm+snip': ('grad_norm', 'snip'), 'jacob_cov': ('jacob_cov',), 'synflow': ('synflow',), 'nwot': ('nwot',),
-          'grad_norm+snip+nwot': ('grad_norm', 'snip', 'nwot')}
+          'grad_norm+snip+nwot': ('grad_norm', 'snip', 'nwot'), 'zico': ('zico',)}
 
 
 def gpu_info():
@@ -62,17 +65,35 @@ def time_measures(arch, precision, reps, B=64, T=500):
     torch.cuda.synchronize()
     res['gate_gram_call'] = e0.elapsed_time(e1) / reps
     res['relu_layers'] = len(pl.gates)
+    # nbasr_grad_snr alone on the model's own N = 2 snapshots (CUDA events)
+    snaps = proxies.zico_snapshots(model, b, 2)
+    names = proxies.scored_names(model)
+    off, ln, chunks, part, out = proxies._segments(eng, names)
+    st = torch.cuda.current_stream().cuda_stream
+
+    def snr():
+        _lib.check(eng.lib.nbasr_grad_snr(snaps.data_ptr(), snaps.stride(0), 2, off.data_ptr(), ln.data_ptr(), len(names),
+                                          chunks, part.data_ptr(), out.data_ptr(), st), 'grad_snr')
+    snr()
+    e0.record()
+    for _ in range(20 * reps):
+        snr()
+    e1.record()
+    torch.cuda.synchronize()
+    res['grad_snr_us'] = e0.elapsed_time(e1) / (20 * reps) * 1e3
+    res['grad_snr_params'] = int(ln.sum())
+    res['grad_snr_GB_per_s'] = 2 * 4 * res['grad_snr_params'] / (res['grad_snr_us'] * 1e3)
     model._engine = None
     return res
 
 
-def sweep_rate(archs, batches, measures):
+def sweep_rate(archs, batches, measures, precision='bf16'):
     kw = dict(proxies=measures, proxy_batches=1) if measures else {}
     n_ref = sum(int(tl.sum()) for _, (t, tl) in batches)
-    sweep.evaluate_arch(archs[0], batches, 0, 'bf16', init='device', conv_gain=101 ** 0.5, n_ref=n_ref, **kw)   # warm-up
+    sweep.evaluate_arch(archs[0], batches, 0, precision, init='device', conv_gain=101 ** 0.5, n_ref=n_ref, **kw)   # warm-up
     torch.cuda.synchronize()
     t0 = time.perf_counter()
-    rows = [sweep.evaluate_arch(a, batches, 0, 'bf16', init='device', conv_gain=101 ** 0.5, n_ref=n_ref, **kw) for a in archs]
+    rows = [sweep.evaluate_arch(a, batches, 0, precision, init='device', conv_gain=101 ** 0.5, n_ref=n_ref, **kw) for a in archs]
     torch.cuda.synchronize()
     dt = time.perf_counter() - t0
     return len(archs) / dt, rows
@@ -100,8 +121,14 @@ def main():
     rn, _ = sweep_rate(archs, batches, ('nwot',))
     r1, rows = sweep_rate(archs, batches, proxies.MEASURES)
     finite = {m: sum(r[m] == r[m] and abs(r[m]) != float('inf') for r in rows) for m in proxies.MEASURES}
+    rz, rows_z = sweep_rate(archs, batches, ('zico',))
+    rz32, rows_z32 = sweep_rate(archs, batches, ('zico',), precision='fp32')
+    z16, z32 = [r['zico'] for r in rows_z], [r['zico'] for r in rows_z32]
+    from scipy.stats import kendalltau
     out['sweep'] = dict(n_archs=len(archs), sample_step=step, archs_per_s=r0, archs_per_s_with_nwot=rn,
                         archs_per_s_with_proxies=r1, measures=list(proxies.MEASURES), rows_with_finite=finite,
+                        archs_per_s_with_zico=rz, archs_per_s_with_zico_fp32=rz32,
+                        zico_kendall_tau_bf16_vs_fp32=float(kendalltau(z16, z32)[0]), zico_bf16=z16, zico_fp32=z32,
                         eval_batches=len(batches), proxy_batches=1)
     print(json.dumps(out['sweep']), flush=True)
     print(json.dumps(dict(gpu=out['gpu'])))
